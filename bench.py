@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the colour-depth pixel-match hot path (BASELINE.json metric: mask x target CDS comparisons / s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1], "1,000 EM masks x 100,000 LM targets pixel-match search, 1210x566, on
@@ -14,6 +14,10 @@ library, per-mask top-K on the device, results on the host.  Inputs are syntheti
 One JSON line on stdout (rank 0).  `value` uses device time (CUDA events on the library's launch stream, summed over the
 step's kernels, max over ranks); `e2e` is wall clock through the C ABI with host buffers (uploads + encoding + mask
 preparation + search + read-back inside the timed region).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0, after the host merge): score, target, mirrored [M, K] and
+count [M] of the per-mask top-K (the --impl reference arm: its dense score and mirrored [M, T]).  The inputs are seeded, so two
+builds run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -584,8 +588,10 @@ def run_reference(args):
         O.search_dense(oms[:4], targets[: max(cores, 8)], cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.search_dense(oms, targets, cores)
+        scores, mirrored, _ = O.search_dense(oms, targets, cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"score": scores, "mirrored": mirrored})
     value = n_m * n_t * args.steps / dt
     sample = "%d masks x %d targets per step (bounded sample of the workload), OpenMP over targets" % (n_m, n_t)
     cfg = workload_config(args, world)
@@ -602,6 +608,25 @@ def run_reference(args):
         "note": "Java reference cannot run here (no JVM); this is the C port of its algorithm pinned on its golden vectors",
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes the last timed step's per-mask result arrays (`name` -> array, one row per mask) as out_dir/<name>.npy in float64,
+    so that two builds can be compared output for output.  When they would exceed DUMP_LIMIT_BYTES, a fixed sample of mask rows
+    (seeded, sorted) is written instead; mask_index.npy always names the rows written."""
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(8 * int(np.prod(a.shape[1:])) for a in arrays.values()) + 8
+    budget = DUMP_LIMIT_BYTES - 1024 * (len(arrays) + 1)          # room for the .npy headers
+    rows = np.arange(n)
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, budget // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "mask_index.npy"), rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a)[rows].astype(np.float64))
 
 
 def workload_config(args, world):
@@ -636,7 +661,10 @@ def main():
     ap.add_argument("--no-pair-provider", action="store_true", help="skip the single-pair (micro-batching queue) leg")
     ap.add_argument("--no-bind", action="store_true", help="do not move the rank onto the CPUs next to its GPU")
     ap.add_argument("--no-data-dependence", action="store_true", help="skip the real-fixture / dense-target legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     if args.impl == "reference":
@@ -706,6 +734,9 @@ def main():
         merged = sharding.gather_and_merge_topk(last, TOPK, t_first)
     elif last is not None:
         merged = last
+    if args.dump_outputs and merged is not None:
+        score, target, mirrored, count = merged
+        dump_outputs(args.dump_outputs, {"score": score, "target": target, "mirrored": mirrored, "count": count})
 
     # max over ranks of the device time
     times = torch.tensor([dev_ms, match_ms, wall_s * 1e3], dtype=torch.float64, device="cuda")
