@@ -55,6 +55,12 @@ class TiffInfo(C.Structure):
                 ("n_strips", C.c_int32), ("big_endian", C.c_int32), ("data_bytes", C.c_int64), ("decodable", C.c_int32), ("pad", C.c_int32)]
 
 
+class TargetGroupsC(C.Structure):
+    """cds_target_groups: group keys of the targets of a best-matches search."""
+    _fields_ = [("line", C.POINTER(C.c_int32)), ("sample", C.POINTER(C.c_int32)), ("line_hash", C.POINTER(C.c_int32)), ("n_lines", C.c_int32),
+                ("sample_hash", C.POINTER(C.c_int32)), ("n_samples", C.c_int32)]
+
+
 _lib = None
 _vp = C.c_void_p
 _u8p = C.POINTER(C.c_uint8)
@@ -122,6 +128,14 @@ SIGNATURES = {
     "cds_normalize_scores": (C.c_int32, [_i32p, _i64p, _i64p, C.c_int64, _f32p]),
     "cds_select_best_matches": (C.c_int32, [_i32p, _i32p, _i32p, C.c_int64, _i32p, C.c_int32, _i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i64p, _i64p]),
     "cds_java_string_hash": (C.c_int32, [C.c_char_p]),
+    "cds_search_best_matches": (C.c_int32, [_vp, _vp, _vp, C.POINTER(TargetGroupsC), C.c_double, C.c_int32, C.c_int32, C.c_int32, C.c_int64,
+                                            _i32p, _i64p, _i32p, _u8p, _i64p]),
+    "cds_search_stream_best_matches_tiff": (C.c_int32, [_vp, _vp, _vp, _i64p, C.c_int64, C.POINTER(TargetGroupsC), C.c_double, C.c_int32, C.c_int32,
+                                                        C.c_int32, C.c_int64, _i32p, _i64p, _i32p, _u8p, _i64p]),
+    "cds_search_stream_best_matches_rgb": (C.c_int32, [_vp, _vp, _vp, C.c_int64, C.POINTER(TargetGroupsC), C.c_double, C.c_int32, C.c_int32,
+                                                       C.c_int32, C.c_int64, _i32p, _i64p, _i32p, _u8p, _i64p]),
+    "cds_debug_select_best_matches_device": (C.c_int32, [_vp, _i32p, _i64p, _i32p, _u8p, C.c_int64, C.POINTER(TargetGroupsC), C.c_int32, C.c_int32,
+                                                         C.c_int32, _i64p, _i64p]),
     "cds_synth_rgb": (C.c_int32, [_vp, C.c_int32, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _vp]),
     "cds_synth_gradient": (C.c_int32, [_vp, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _vp]),
     "cds_get_last_stats": (C.c_int32, [_vp, C.POINTER(SearchStats)]),
@@ -525,6 +539,46 @@ class MaskSet:
             return mask[:c], target[:c], score[:c], mir[:c]
         _check(st, self.ctx.h)
 
+    def _best_matches(self, call, capacity):
+        """Runs call(capacity, mask, target, score, mirrored, count) of a *_best_matches entry; with capacity=None it is retried once with
+        the number of selected pairs the library reports."""
+        cap = int(capacity) if capacity is not None else max(1024, 4 * len(self))
+        for _ in range(2):
+            mask = np.zeros(cap, np.int32); target = np.zeros(cap, np.int64); score = np.zeros(cap, np.int32); mir = np.zeros(cap, np.uint8)
+            count = C.c_int64(0)
+            st = call(cap, mask.ctypes.data_as(_i32p), target.ctypes.data_as(_i64p), score.ctypes.data_as(_i32p), mir.ctypes.data_as(_u8p),
+                      C.byref(count))
+            if st == CDS_ERR_CAPACITY and capacity is None and count.value > cap:
+                cap = int(count.value)
+                continue
+            _check(st, self.ctx.h)
+            c = int(count.value)
+            return mask[:c], target[:c], score[:c], mir[:c]
+        _check(st, self.ctx.h)
+
+    def search_best_matches(self, library, groups, pct_positive_pixels, top_lines, top_samples, top_matches, capacity=None):
+        """cds_search_best_matches: per mask, the pairs ColorMIPProcessUtils.selectBestMatches keeps, selected on the device ->
+        (mask, target, score, mirrored) arrays.  groups: TargetGroups indexed by library index."""
+        g = groups.struct()
+        return self._best_matches(lambda cap, *out: lib().cds_search_best_matches(
+            self.ctx.h, self.h, library.h, C.byref(g), float(pct_positive_pixels), int(top_lines), int(top_samples), int(top_matches), cap, *out), capacity)
+
+    def search_stream_best_matches_tiff(self, files, groups, pct_positive_pixels, top_lines, top_samples, top_matches, capacity=None):
+        """cds_search_stream_best_matches_tiff: the same over TIFF files in host memory (groups indexed by file)."""
+        blob, offsets = pack_files(files)
+        g = groups.struct()
+        return self._best_matches(lambda cap, *out: lib().cds_search_stream_best_matches_tiff(
+            self.ctx.h, self.h, _ptr(blob), offsets.ctypes.data_as(_i64p), len(offsets) - 1, C.byref(g), float(pct_positive_pixels),
+            int(top_lines), int(top_samples), int(top_matches), cap, *out), capacity)
+
+    def search_stream_best_matches_rgb(self, targets_rgb, groups, pct_positive_pixels, top_lines, top_samples, top_matches, capacity=None):
+        """cds_search_stream_best_matches_rgb: the same over RGB images in host memory (groups indexed by image)."""
+        targets_rgb = np.ascontiguousarray(targets_rgb, dtype=np.uint8)
+        g = groups.struct()
+        return self._best_matches(lambda cap, *out: lib().cds_search_stream_best_matches_rgb(
+            self.ctx.h, self.h, _ptr(targets_rgb), int(targets_rgb.shape[0]), C.byref(g), float(pct_positive_pixels),
+            int(top_lines), int(top_samples), int(top_matches), cap, *out), capacity)
+
     def score_pair(self, mask_index, target_rgb):
         target_rgb = np.ascontiguousarray(target_rgb, dtype=np.uint8)
         s = C.c_int32()
@@ -846,18 +900,57 @@ def java_string_hash(s):
     return int(lib().cds_java_string_hash(s.encode("ascii")))
 
 
+def _group_ids(keys):
+    """key strings -> (dense ids in first-appearance order, Java hashCode() per id); blank keys count as "UNKNOWN"."""
+    table, out = {}, []
+    for k in keys:
+        k = k if k and k.strip() else "UNKNOWN"            # StringUtils.defaultIfBlank
+        out.append(table.setdefault(k, len(table)))
+    names = sorted(table, key=table.get)
+    return np.asarray(out, np.int32), np.asarray([java_string_hash(nm) for nm in names], np.int32)
+
+
+class TargetGroups:
+    """The group keys of the targets of a best-matches search (cds_target_groups): lines[i] / samples[i] = published name / neuron id
+    of target i, as strings; ids and hashes are derived the way select_best_matches derives them."""
+
+    def __init__(self, lines, samples):
+        self.line, self.line_hash = _group_ids(lines)
+        self.sample, self.sample_hash = _group_ids(samples)
+        if len(self.line) != len(self.sample):
+            raise ValueError("lines and samples must name the same targets")
+
+    def __len__(self):
+        return len(self.line)
+
+    def struct(self):
+        """The C struct; it points into this object's arrays, so keep the object alive while the struct is used."""
+        def p(a):
+            return a.ctypes.data_as(_i32p) if len(a) else None
+        return TargetGroupsC(p(self.line), p(self.sample), p(self.line_hash), len(self.line_hash), p(self.sample_hash), len(self.sample_hash))
+
+
+def debug_select_best_matches_device(ctx, mask, target, score, mirrored, groups, top_lines, top_samples_per_line, top_matches_per_sample):
+    """cds_debug_select_best_matches_device: the device selection alone over a list sorted by (mask, score desc, target asc);
+    returns indices into the list in output order."""
+    mask = np.ascontiguousarray(mask, np.int32); target = np.ascontiguousarray(target, np.int64); score = np.ascontiguousarray(score, np.int32)
+    mirrored = None if mirrored is None else np.ascontiguousarray(mirrored, np.uint8)
+    n = len(mask)
+    sel = np.zeros(max(n, 1), np.int64)
+    cnt = C.c_int64(0)
+    g = groups.struct()
+    _check(lib().cds_debug_select_best_matches_device(ctx.h, mask.ctypes.data_as(_i32p), target.ctypes.data_as(_i64p), score.ctypes.data_as(_i32p),
+                                                      None if mirrored is None else mirrored.ctypes.data_as(_u8p), n, C.byref(g), int(top_lines),
+                                                      int(top_samples_per_line), int(top_matches_per_sample), sel.ctypes.data_as(_i64p),
+                                                      C.byref(cnt)), ctx.h)
+    return sel[: cnt.value]
+
+
 def select_best_matches(lines, samples, scores, top_lines, top_samples_per_line, top_matches_per_sample):
     """ColorMIPProcessUtils.selectBestMatches over one mask's matches.  lines / samples: sequences of key strings (ASCII);
     returns the indices of the kept matches in the reference's output order."""
-    def ids(keys):
-        table, out = {}, []
-        for k in keys:
-            k = k if k and k.strip() else "UNKNOWN"            # StringUtils.defaultIfBlank
-            out.append(table.setdefault(k, len(table)))
-        names = sorted(table, key=table.get)
-        return np.asarray(out, np.int32), np.asarray([java_string_hash(nm) for nm in names], np.int32)
-    lid, lhash = ids(lines)
-    sid, shash = ids(samples)
+    lid, lhash = _group_ids(lines)
+    sid, shash = _group_ids(samples)
     sc = np.ascontiguousarray(scores, np.int32)
     n = len(sc)
     sel = np.zeros(max(n, 1), np.int64)

@@ -362,6 +362,11 @@ extern "C" cds_status cds_ctx_set_option(cds_ctx *ctx, const char *name, int64_t
             ctx->stream_chunk_tiff = value;
             return CDS_OK;
         }
+        if (std::strcmp(name, "best_list_bytes") == 0) {
+            if (value < 12 || value > ((int64_t) 4 << 30)) return ctx->fail(CDS_ERR_BAD_ARG, "cds_ctx_set_option: best_list_bytes must be 12..4294967296");
+            ctx->best_list_bytes = value;
+            return CDS_OK;
+        }
         if (std::strcmp(name, "fused_ingest") == 0) { ctx->fused_ingest = value != 0; return CDS_OK; }
         if (std::strcmp(name, "cand_wait_mode") == 0) { cand_tuning().wait_mode = (int) value; return CDS_OK; }
         if (std::strcmp(name, "cand_l2_hint") == 0) { cand_tuning().l2_hint = value != 0; return CDS_OK; }

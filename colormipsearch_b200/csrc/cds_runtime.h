@@ -122,6 +122,7 @@ struct cds_ctx {
     int fused_ingest = 1;         // cds_ctx_set_option("fused_ingest"): 1 = TIFF strips go straight to code words (tiff_encode_kernel), 0 = decode to RGB, then encode
     int64_t stream_chunk_bytes = 0xC0000000ll;   // cds_ctx_set_option("stream_chunk_bytes"): most file bytes per chunk (the strip table addresses them with 32 bits)
     int64_t stream_chunk_tiff = 4096;   // cds_ctx_set_option("stream_chunk_tiff"): targets per chunk of cds_search_stream_tiff
+    int64_t best_list_bytes = (int64_t) 1 << 30;   // cds_ctx_set_option("best_list_bytes"): per-device list of passing pairs of the *_best_matches searches
 
     cds_status fail(cds_status code, const std::string &msg) const;
     cds_status check(cudaError_t e, const char *what) const;

@@ -16,6 +16,7 @@
 
 #include "cds_runtime.h"
 #include "cds_band.cuh"
+#include "cds_bestsel.cuh"
 #include "cds_topk.cuh"
 #include "cds_tiff.h"
 
@@ -232,16 +233,30 @@ struct AllMatchesOut {
     int64_t *count;
 };
 
+// The third mode: the passing pairs stay on the devices (within "best_list_bytes" per device) and only the best-matches selection
+// over them (csrc/cds_bestsel.cu) comes back.
+struct BestMatchesOut {
+    const cds_target_groups *groups;
+    int32_t top_lines, top_samples_per_line, top_matches_per_sample;
+    int64_t capacity;
+    int32_t *mask;
+    int64_t *target;
+    int32_t *score;
+    uint8_t *mirrored;
+    int64_t *count;
+};
+
 cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8_t *targets_rgb, int64_t n_targets,
                               int32_t k, double pct_positive_pixels,
                               int32_t *out_score, int64_t *out_target, uint8_t *out_mirrored, int32_t *out_count, const AllMatchesOut *all,
-                              cds_library *resident, const TiffSource *tiff = nullptr)
+                              cds_library *resident, const TiffSource *tiff = nullptr, const BestMatchesOut *best = nullptr)
 {
     std::lock_guard<std::recursive_mutex> lk(ctx->mu);
     cds_maskset *ms = const_cast<cds_maskset *>(ms_c);
     if (ms->ctx != ctx) return ctx->fail(CDS_ERR_BAD_ARG, "mask set belongs to another context");
-    if (!all && (k <= 0 || k > topk_max_k())) return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_rgb: k must be in 1..4096");
-    if (all) k = 1;
+    const bool collect = all || best;      // every passing pair goes to a device list
+    if (!collect && (k <= 0 || k > topk_max_k())) return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_rgb: k must be in 1..4096");
+    if (collect) k = 1;
     if (resident) n_targets = resident->size;
     if (!resident && !tiff && (n_targets < 0 || (n_targets > 0 && !targets_rgb))) return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_rgb: bad target array");
     if (tiff && (n_targets < 0 || (n_targets > 0 && (!tiff->blob || !tiff->offsets)))) return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_tiff: bad target array");
@@ -251,10 +266,15 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
             return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_matches_rgb: bad output arrays");
         *all->count = 0;
     }
+    if (best) {
+        if (!best->count || best->capacity < 0 || (best->capacity > 0 && (!best->mask || !best->target || !best->score)))
+            return ctx->fail(CDS_ERR_BAD_ARG, "best matches: bad output arrays");
+        *best->count = 0;
+    }
     if (M == 0) return CDS_OK;
-    if (!all && (!out_score || !out_target || !out_count)) return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_rgb: NULL output");
+    if (!collect && (!out_score || !out_target || !out_count)) return ctx->fail(CDS_ERR_BAD_ARG, "cds_search_stream_rgb: NULL output");
     ctx->stats = cds_search_stats{};
-    if (!all) for (int m = 0; m < M; m++) out_count[m] = 0;
+    if (!collect) for (int m = 0; m < M; m++) out_count[m] = 0;
     if (n_targets == 0) return CDS_OK;
     // A mask set that has changed since its last search still needs its palettes and word lists (sync_descs: a few small kernels and
     // several host round trips, ~3 ms for 1 000 masks).  The search over files does not wait for that: the first chunk's upload, ingest
@@ -308,17 +328,23 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
     std::vector<int32_t> min_score(M);
     for (int m = 0; m < M; m++) min_score[m] = min_matching_score(ms->sizes[m], pct_positive_pixels);
     const int used_devs = resident ? D : (int) std::min<int64_t>(D, n_chunks);
+    // entries of a device's list of passing pairs
+    const int64_t list_cap = best ? ctx->best_list_bytes / kBestPairBytes : all ? all->capacity : 0;
     std::vector<uint64_t *> all_keys(D, nullptr);
     std::vector<int32_t *> all_masks(D, nullptr);
     std::vector<unsigned long long *> all_counter(D, nullptr);
+    std::vector<DevGroups> groups(D);          // best: the targets' group keys on every device
+    std::vector<void *> gathered;              // best, several devices: the lists moved to the first device
     auto release_all = [&]() {
         for (int d = 0; d < D; d++) {
-            if (!all_keys[d] && !all_masks[d] && !all_counter[d]) continue;
+            if (!all_keys[d] && !all_masks[d] && !all_counter[d] && !groups[d].line && !(d == 0 && !gathered.empty())) continue;
             cudaSetDevice(ctx->devs[d].dev);
             cudaStreamSynchronize(ctx->devs[d].stream);
             ctx->devs[d].pool.free(all_keys[d]);
             ctx->devs[d].pool.free(all_masks[d]);
             ctx->devs[d].pool.free(all_counter[d]);
+            groups[d].release(ctx->devs[d]);
+            if (d == 0) for (void *p : gathered) ctx->devs[0].pool.free(p);
         }
     };
     struct Releaser { std::function<void()> f; ~Releaser() { f(); } } releaser{release_all};
@@ -328,8 +354,9 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
         if (tiff) CDS_TRY(ensure_tiff_bufs(ctx, ds, tiff_comp_bytes, (size_t) chunk * 128));
         CDS_CUDA(ctx, cudaMemcpyAsync(ds.sb.min_score, min_score.data(), (size_t) M * sizeof(int32_t), cudaMemcpyHostToDevice, ds.stream));
         CDS_CUDA(ctx, cudaMemsetAsync(ds.sb.counts_run, 0, (size_t) M * sizeof(int32_t), ds.stream));
-        if (all) {
-            const size_t cap = (size_t) std::max<int64_t>(all->capacity, 1);
+        if (best) CDS_TRY(upload_target_groups(ctx, ds, best->groups, n_targets, groups[d]));
+        if (collect) {
+            const size_t cap = (size_t) std::max<int64_t>(list_cap, 1);
             CDS_CUDA(ctx, ds.pool.alloc((void **) &all_keys[d], cap * sizeof(uint64_t)));
             CDS_CUDA(ctx, ds.pool.alloc((void **) &all_masks[d], cap * sizeof(int32_t)));
             CDS_CUDA(ctx, ds.pool.alloc((void **) &all_counter[d], sizeof(unsigned long long)));
@@ -368,6 +395,47 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
         if (!tr) return;
         cudaEventCreate(&tr->ev[i]);
         cudaEventRecord(tr->ev[i], st);
+    };
+
+    // best, with a per-sample limit: a device's list is compacted exactly (bestsel_compact) when the next chunk might not fit.  bound[d]
+    // = most pairs the list can hold by now (a chunk adds at most masks x targets); only when it passes the budget does the host wait
+    // for the true count.  Without a limit the list cannot shrink and a list that overflows fails at the end, with the size it needs.
+    std::vector<int64_t> bound(D, 0), compacted_at(D, -1);
+    auto read_count = [&](int d, int64_t &n) -> cds_status {
+        unsigned long long c = 0;
+        CDS_CUDA(ctx, cudaMemcpyAsync(&c, all_counter[d], sizeof c, cudaMemcpyDeviceToHost, ctx->devs[d].stream));
+        CDS_CUDA(ctx, cudaStreamSynchronize(ctx->devs[d].stream));
+        ctx->stats.d2h_bytes += (int64_t) sizeof c;
+        n = (int64_t) c;
+        return CDS_OK;
+    };
+    auto best_make_room = [&](int d, int64_t most) -> cds_status {
+        if (bound[d] + most <= list_cap) return CDS_OK;
+        int64_t n = 0;
+        CDS_TRY(read_count(d, n));
+        if (n + most > list_cap && n != compacted_at[d]) {
+            // a resident library's keys are still shard-local here
+            CDS_TRY(bestsel_compact(ctx, ctx->devs[d], all_keys[d], all_masks[d], n, all_counter[d], groups[d], best->top_matches_per_sample,
+                                    resident ? d : 0, resident ? D : 1));
+            compacted_at[d] = n;
+            CDS_CUDA(ctx, cudaSetDevice(ctx->devs[d].dev));
+        }
+        bound[d] = n;
+        return CDS_OK;
+    };
+    auto best_check = [&](int d, int64_t most) -> cds_status {
+        bound[d] += most;
+        if (bound[d] <= list_cap) return CDS_OK;
+        int64_t n = 0;
+        CDS_TRY(read_count(d, n));
+        if (n > list_cap) {
+            char buf[300];
+            snprintf(buf, sizeof buf, "best matches: the passing pairs of device %d need at least %lld bytes after keeping %d per sample; "
+                     "\"best_list_bytes\" is %lld", d, (long long) (n * kBestPairBytes), best->top_matches_per_sample, (long long) ctx->best_list_bytes);
+            return ctx->fail(CDS_ERR_CAPACITY, buf);
+        }
+        bound[d] = n;
+        return CDS_OK;
     };
 
     // enqueue every chunk; nothing below blocks the host when the source is pinned memory
@@ -460,10 +528,13 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
         }
         if (tr && tiff) mark(tr, 3, ds.stream);
         CDS_TRY(launch_match_view(ctx, ms, tv, d, 0, M, sb.scores, ds.stream, sb.timing[2 * j], sb.timing[2 * j + 1]));
-        if (all) {
+        if (collect) {
+            const bool compacting = best && best->top_matches_per_sample > 0;
+            if (compacting) CDS_TRY(best_make_room(d, (int64_t) M * cnt));
             launch_collect_matches(sb.scores, M, cnt, sb.min_score, 0, first, all_keys[d], all_masks[d], all_counter[d],
-                                   (unsigned long long) all->capacity, ds.stream);
+                                   (unsigned long long) list_cap, ds.stream);
             ctx->stats.kernel_launches++;
+            if (compacting) CDS_TRY(best_check(d, (int64_t) M * cnt));
         } else {
             launch_topk(sb.scores, M, cnt, sb.min_score, k, first, sb.keys_chunk, sb.counts_chunk, ds.stream);
             launch_topk_merge(sb.keys_run, sb.counts_run, sb.keys_chunk, sb.counts_chunk, M, k, ds.stream);
@@ -480,7 +551,7 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
         DevState &ds = ctx->devs[d];
         CDS_CUDA(ctx, cudaSetDevice(ds.dev));
         CDS_CUDA(ctx, cudaEventRecord(ds.ev2, ds.stream));
-        if (all) {
+        if (collect) {
             CDS_CUDA(ctx, cudaMemcpyAsync(&all_n[d], all_counter[d], sizeof(unsigned long long), cudaMemcpyDeviceToHost, ds.stream));
             continue;
         }
@@ -527,6 +598,82 @@ cds_status stream_search_impl(cds_ctx *ctx, const cds_maskset *ms_c, const uint8
     ctx->stats.total_device_ms = total_ms;
     ctx->stats.comparisons = (int64_t) M * n_targets;
     ctx->stats.chunked = 1;
+    if (best) {
+        // the selection runs where all of a mask's pairs are: the first device; only the selected pairs and their count come back
+        std::vector<int64_t> n_dev(used_devs);
+        for (int d = 0; d < used_devs; d++) {
+            ctx->stats.d2h_bytes += (int64_t) sizeof(unsigned long long);
+            n_dev[d] = (int64_t) all_n[d];
+            if (n_dev[d] > list_cap) {
+                char buf[300];
+                snprintf(buf, sizeof buf, "best matches: %lld pairs pass isMatch on device %d, their list needs %lld bytes; \"best_list_bytes\" is %lld%s",
+                         (long long) n_dev[d], d, (long long) (n_dev[d] * kBestPairBytes), (long long) ctx->best_list_bytes,
+                         best->top_matches_per_sample > 0 ? "" : " (without a per-sample limit the list cannot be compacted)");
+                return ctx->fail(CDS_ERR_CAPACITY, buf);
+            }
+        }
+        for (int d = 0; d < used_devs; d++) {
+            DevState &ds = ctx->devs[d];
+            CDS_CUDA(ctx, cudaSetDevice(ds.dev));
+            if (resident) launch_bestsel_globalize(all_keys[d], n_dev[d], d, D, ds.stream);
+            CDS_CUDA(ctx, cudaGetLastError());
+            if (used_devs > 1)
+                CDS_TRY(bestsel_compact(ctx, ds, all_keys[d], all_masks[d], n_dev[d], all_counter[d], groups[d], best->top_matches_per_sample, 0, 1));
+        }
+        DevState &d0 = ctx->devs[0];
+        uint64_t *keys = all_keys[0];
+        int32_t *masks = all_masks[0];
+        int64_t n = n_dev[0];
+        if (used_devs > 1) {
+            for (int d = 1; d < used_devs; d++) n += n_dev[d];
+            for (int d = 0; d < used_devs; d++) {
+                CDS_CUDA(ctx, cudaSetDevice(ctx->devs[d].dev));
+                CDS_CUDA(ctx, cudaStreamSynchronize(ctx->devs[d].stream));
+            }
+            CDS_CUDA(ctx, cudaSetDevice(d0.dev));
+            void *gk = nullptr, *gm = nullptr;
+            CDS_CUDA(ctx, d0.pool.alloc(&gk, (size_t) std::max<int64_t>(n, 1) * sizeof(uint64_t)));
+            gathered.push_back(gk);
+            CDS_CUDA(ctx, d0.pool.alloc(&gm, (size_t) std::max<int64_t>(n, 1) * sizeof(int32_t)));
+            gathered.push_back(gm);
+            keys = (uint64_t *) gk;
+            masks = (int32_t *) gm;
+            int64_t at = 0;
+            for (int d = 0; d < used_devs; d++) {
+                DevState &src = ctx->devs[d];
+                const struct { void *dst; const void *src; size_t bytes; } parts[] = {
+                    {keys + at, all_keys[d], (size_t) n_dev[d] * sizeof(uint64_t)}, {masks + at, all_masks[d], (size_t) n_dev[d] * sizeof(int32_t)}};
+                at += n_dev[d];
+                int peer = 0;
+                if (src.dev != d0.dev) CDS_CUDA(ctx, cudaDeviceCanAccessPeer(&peer, d0.dev, src.dev));
+                for (const auto &pt : parts) {
+                    if (pt.bytes == 0) continue;
+                    if (src.dev == d0.dev) {
+                        CDS_CUDA(ctx, cudaMemcpyAsync(pt.dst, pt.src, pt.bytes, cudaMemcpyDeviceToDevice, d0.stream));
+                    } else if (peer) {
+                        CDS_CUDA(ctx, cudaMemcpyPeerAsync(pt.dst, d0.dev, pt.src, src.dev, pt.bytes, d0.stream));
+                    } else {
+                        // no peer access: staged through pinned host memory
+                        CDS_TRY(ctx->ensure_pinned(src, pt.bytes));
+                        CDS_CUDA(ctx, cudaSetDevice(src.dev));
+                        CDS_CUDA(ctx, cudaMemcpyAsync(src.h_pinned, pt.src, pt.bytes, cudaMemcpyDeviceToHost, src.stream));
+                        CDS_CUDA(ctx, cudaStreamSynchronize(src.stream));
+                        CDS_CUDA(ctx, cudaSetDevice(d0.dev));
+                        CDS_CUDA(ctx, cudaMemcpyAsync(pt.dst, src.h_pinned, pt.bytes, cudaMemcpyHostToDevice, d0.stream));
+                        CDS_CUDA(ctx, cudaStreamSynchronize(d0.stream));
+                        ctx->stats.d2h_bytes += (int64_t) pt.bytes;
+                        ctx->stats.h2d_bytes += (int64_t) pt.bytes;
+                    }
+                }
+            }
+        }
+        BestSelOut o;
+        o.capacity = best->capacity;
+        o.mask = best->mask; o.target = best->target; o.score = best->score; o.mirrored = best->mirrored;
+        o.count = best->count;
+        return bestsel_select(ctx, d0, keys, masks, n, M, false, groups[0], best->top_lines, best->top_samples_per_line,
+                              best->top_matches_per_sample, o);
+    }
     if (all) {
         // every passing pair, ordered like the reference's writer: by mask, descending matchingPixels, ascending target
         uint64_t total = 0;
@@ -673,5 +820,71 @@ extern "C" cds_status cds_search_matches(cds_ctx *ctx, const cds_maskset *ms, cd
         }
         const AllMatchesOut all{capacity, out_mask, out_target, out_score, out_mirrored, out_count};
         return stream_search_impl(ctx, ms, nullptr, 0, 1, pct_positive_pixels, nullptr, nullptr, nullptr, nullptr, &all, lib);
+    });
+}
+
+// The best-matches searches: the same collection of passing pairs, then ColorMIPProcessUtils.selectBestMatches per mask on the
+// device (csrc/cds_bestsel.cu).  The groups are checked before anything touches a device.
+namespace {
+cds_status best_matches_entry(const char *name, cds_ctx *ctx, const cds_maskset *ms, int64_t n_targets, const cds_target_groups *groups,
+                              const std::function<cds_status()> &run)
+{
+    const std::string err = cds::check_target_groups(groups, std::max<int64_t>(n_targets, 0));
+    if (!err.empty()) {
+        if (!ctx) { set_tls_error(std::string(name) + ": " + err); return CDS_ERR_BAD_ARG; }
+        std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+        return ctx->fail(CDS_ERR_BAD_ARG, std::string(name) + ": " + err);
+    }
+    if (!ctx || !ms) { set_tls_error(std::string(name) + ": NULL argument"); return CDS_ERR_BAD_ARG; }
+    return run();
+}
+}  // namespace
+
+extern "C" cds_status cds_search_best_matches(cds_ctx *ctx, const cds_maskset *ms, cds_library *lib, const cds_target_groups *groups,
+                                              double pct_positive_pixels, int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
+                                              int64_t capacity, int32_t *out_mask, int64_t *out_target, int32_t *out_score, uint8_t *out_mirrored,
+                                              int64_t *out_count)
+{
+    return cds::abi_guard("cds_search_best_matches", [&]() -> cds_status {
+        if (!lib) { set_tls_error("cds_search_best_matches: NULL argument"); return CDS_ERR_BAD_ARG; }
+        return best_matches_entry("cds_search_best_matches", ctx, ms, lib->size, groups, [&]() -> cds_status {
+            if (ms->W != lib->g.W || ms->H != lib->g.H) {
+                std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+                char buf[200];
+                snprintf(buf, sizeof buf, "Invalid image size - target's image size (%d, %d) must match query's image size: (%d, %d)", ms->W, ms->H, lib->g.W, lib->g.H);
+                return ctx->fail(CDS_ERR_SIZE_MISMATCH, buf);
+            }
+            const BestMatchesOut best{groups, top_lines, top_samples_per_line, top_matches_per_sample, capacity, out_mask, out_target, out_score, out_mirrored, out_count};
+            return stream_search_impl(ctx, ms, nullptr, 0, 1, pct_positive_pixels, nullptr, nullptr, nullptr, nullptr, nullptr, lib, nullptr, &best);
+        });
+    });
+}
+
+extern "C" cds_status cds_search_stream_best_matches_tiff(cds_ctx *ctx, const cds_maskset *ms, const uint8_t *blob, const int64_t *offsets,
+                                                          int64_t n_targets, const cds_target_groups *groups, double pct_positive_pixels,
+                                                          int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
+                                                          int64_t capacity, int32_t *out_mask, int64_t *out_target, int32_t *out_score,
+                                                          uint8_t *out_mirrored, int64_t *out_count)
+{
+    return cds::abi_guard("cds_search_stream_best_matches_tiff", [&]() -> cds_status {
+        return best_matches_entry("cds_search_stream_best_matches_tiff", ctx, ms, n_targets, groups, [&]() -> cds_status {
+            const BestMatchesOut best{groups, top_lines, top_samples_per_line, top_matches_per_sample, capacity, out_mask, out_target, out_score, out_mirrored, out_count};
+            const TiffSource src{blob, offsets};
+            return stream_search_impl(ctx, ms, nullptr, n_targets, 1, pct_positive_pixels, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, &src, &best);
+        });
+    });
+}
+
+extern "C" cds_status cds_search_stream_best_matches_rgb(cds_ctx *ctx, const cds_maskset *ms, const uint8_t *targets_rgb, int64_t n_targets,
+                                                         const cds_target_groups *groups, double pct_positive_pixels,
+                                                         int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
+                                                         int64_t capacity, int32_t *out_mask, int64_t *out_target, int32_t *out_score,
+                                                         uint8_t *out_mirrored, int64_t *out_count)
+{
+    return cds::abi_guard("cds_search_stream_best_matches_rgb", [&]() -> cds_status {
+        return best_matches_entry("cds_search_stream_best_matches_rgb", ctx, ms, n_targets, groups, [&]() -> cds_status {
+            const BestMatchesOut best{groups, top_lines, top_samples_per_line, top_matches_per_sample, capacity, out_mask, out_target, out_score, out_mirrored, out_count};
+            return stream_search_impl(ctx, ms, targets_rgb, n_targets, 1, pct_positive_pixels, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, &best);
+        });
     });
 }

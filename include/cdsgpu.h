@@ -111,6 +111,10 @@ int32_t    cds_abi_version(void);
  * "wide_lists": 1 = mask sets prepared from now on carry each mask pixel's rank interval in the candidate kernel's lists (4 bytes per
  *   pixel and list) instead of a reference into a per-group palette (2 bytes).  0 (default): only sets with a group of more than
  *   2 047 colour classes do (brightness-scaled LM images as masks -- the reverse search); scores are the same either way.
+ * "best_list_bytes": most bytes per device of the list of passing pairs that the *_best_matches searches keep on the device (12 bytes per
+ *   pair; default 1 GiB, 12 .. 4 GiB).  While it runs, the selection over the list takes about 144 bytes more per pair on the first device
+ *   (all devices' lists together) and a compaction about 96; a call that would not fit in the device's free memory returns CDS_ERR_OOM
+ *   naming the bytes it needs.
  * Unknown names: CDS_ERR_BAD_ARG. */
 cds_status cds_ctx_set_option(cds_ctx *ctx, const char *name, int64_t value);
 
@@ -411,6 +415,63 @@ cds_status cds_select_best_matches(const int32_t *line, const int32_t *sample, c
                                    const int32_t *line_hash, int32_t n_lines, const int32_t *sample_hash, int32_t n_samples,
                                    int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
                                    int64_t *selected, int64_t *n_selected);
+/* The same selection fused into the searches, on the device (csrc/cds_bestsel.cu): what the reference's two steps keep -- colorDepthSearch
+ * writes every pair that passes isMatch, gradientScores reads them back and keeps ColorMIPProcessUtils.selectBestMatches
+ * (TOOLS/cdsprocess/ColorMIPProcessUtils.java:12-34, API/results/ItemsHandling.java:80-109) per mask -- without the passing pairs
+ * crossing PCIe.  Group keys of the targets are indexed like the targets of the search (library index, or file / image index of a
+ * streamed call); every id must lie in [0, n_lines) / [0, n_samples). */
+typedef struct cds_target_groups {
+    const int32_t *line;          /* [n_targets] dense id of the target's published name (blank -> "UNKNOWN" mapped by the caller) */
+    const int32_t *sample;        /* [n_targets] dense id of the neuron id / sample */
+    const int32_t *line_hash;     /* [n_lines]   Java String.hashCode() of each line key */
+    int32_t        n_lines;
+    const int32_t *sample_hash;   /* [n_samples] Java String.hashCode() of each sample key */
+    int32_t        n_samples;
+} cds_target_groups;
+
+/* Per mask, the pairs of cds_search_matches (same pct_positive_pixels) that cds_select_best_matches keeps, in its output order, masks
+ * ascending: the output equals, bit for bit and in the same order, cds_search_matches followed by cds_select_best_matches over each
+ * mask's slice (which is already in the reference's encounter order, score descending, then target ascending) with the targets' group
+ * ids and hashes.  As a restatement that sorting computes: per (mask, line), best = its highest score and first = the smallest target
+ * among its pairs with that score (its first appearance); cap = 16, doubled while the mask's number of distinct lines > 0.75 * cap;
+ * bucket = (h ^ (h >>> 16)) & (cap - 1) of the line's hash h.  Lines are ranked by (best desc, bucket asc, first asc) and the first
+ * top_lines kept.  Inside a kept line the samples are ranked the same way, cap counting the distinct samples of that line (the
+ * reference builds one HashMap per line), and the first top_samples_per_line kept; inside a kept sample the first
+ * top_matches_per_sample pairs in encounter order.  Output order: line rank, sample rank, encounter order.  HashMap tree bins are
+ * not modelled, as in cds_select_best_matches.
+ * top_* <= 0 mean "no limit".  out_* hold `capacity` entries; *out_count receives the number selected; when more are selected than
+ * `capacity`, nothing is written, *out_count still tells how many and the call returns CDS_ERR_CAPACITY.  CDS_ERR_SIZE_MISMATCH as
+ * cds_search_matches; CDS_ERR_BAD_ARG for a NULL groups or an id outside its range (checked before a device is touched).
+ * The passing pairs are kept on the devices, at most "best_list_bytes" per device (cds_ctx_set_option).  When a list fills and
+ * top_matches_per_sample > 0 it is compacted to the first top_matches_per_sample pairs of every (mask, line, sample), which changes no
+ * selection (every present sample keeps its best pair, so best / first of lines and samples and the numbers of distinct lines and
+ * samples stay); when it still does not fit, or top_matches_per_sample <= 0, the call returns CDS_ERR_CAPACITY naming the bytes needed.
+ * On a context of several devices the lists are moved to the first device (peer copies, staged through pinned host memory where
+ * peer access is missing) and selected there.  Only the selected pairs and their count cross to the host (cds_search_stats.d2h_bytes).
+ * One process per GPU (colormipsearch_b200/sharding.py) does NOT give an exact selection -- a mask's pairs would have to meet from
+ * every rank; use one context over the devices instead. */
+cds_status cds_search_best_matches(cds_ctx *ctx, const cds_maskset *ms, cds_library *lib, const cds_target_groups *groups,
+                                   double pct_positive_pixels, int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
+                                   int64_t capacity, int32_t *out_mask, int64_t *out_target, int32_t *out_score, uint8_t *out_mirrored,
+                                   int64_t *out_count);
+/* The same over TIFF files / RGB images in host memory (targets as in cds_search_stream_matches_tiff / _rgb). */
+cds_status cds_search_stream_best_matches_tiff(cds_ctx *ctx, const cds_maskset *ms, const uint8_t *blob, const int64_t *offsets,
+                                               int64_t n_targets, const cds_target_groups *groups, double pct_positive_pixels,
+                                               int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
+                                               int64_t capacity, int32_t *out_mask, int64_t *out_target, int32_t *out_score,
+                                               uint8_t *out_mirrored, int64_t *out_count);
+cds_status cds_search_stream_best_matches_rgb(cds_ctx *ctx, const cds_maskset *ms, const uint8_t *targets_rgb, int64_t n_targets,
+                                              const cds_target_groups *groups, double pct_positive_pixels,
+                                              int32_t top_lines, int32_t top_samples_per_line, int32_t top_matches_per_sample,
+                                              int64_t capacity, int32_t *out_mask, int64_t *out_target, int32_t *out_score,
+                                              uint8_t *out_mirrored, int64_t *out_count);
+/* Test hook: the device selection alone, on the context's first device, over a caller-given list of one or more masks' passing pairs
+ * sorted by (mask, score desc, target asc) (CDS_ERR_BAD_ARG otherwise); groups are indexed by target.  selected[] (room for n)
+ * receives indices into that list in output order; *n_selected their number. */
+cds_status cds_debug_select_best_matches_device(cds_ctx *ctx, const int32_t *mask, const int64_t *target, const int32_t *score,
+                                                const uint8_t *mirrored, int64_t n, const cds_target_groups *groups, int32_t top_lines,
+                                                int32_t top_samples_per_line, int32_t top_matches_per_sample, int64_t *selected,
+                                                int64_t *n_selected);
 /* java.lang.String.hashCode() of an ASCII string (helper for non-Java callers of cds_select_best_matches). */
 int32_t cds_java_string_hash(const char *ascii);
 

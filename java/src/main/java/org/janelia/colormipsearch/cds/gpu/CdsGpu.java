@@ -62,6 +62,10 @@ public final class CdsGpu {
     public static final MethodHandle libraryAddTiff = h("cds_library_add_tiff", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
     public static final MethodHandle searchStreamTiff = h("cds_search_stream_tiff", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_DOUBLE, ADDRESS, ADDRESS, ADDRESS, ADDRESS));
     public static final MethodHandle searchStreamMatchesTiff = h("cds_search_stream_matches_tiff", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_DOUBLE, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS));
+    // cds_search_best_matches(ctx, maskset, library, const cds_target_groups *groups, pct, topLines, topSamplesPerLine, topMatchesPerSample,
+    //                         capacity, outMask, outTarget, outScore, outMirrored, outCount): selectBestMatches fused into the search, on the
+    // device.  cds_target_groups = {int *line, int *sample, int *lineHash, int nLines, int *sampleHash, int nSamples} (natural C layout, 48 bytes).
+    public static final MethodHandle searchBestMatches = h("cds_search_best_matches", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_DOUBLE, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS));
     public static final MethodHandle shapeScorePairsTiff = h("cds_shape_score_pairs_tiff", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS));
     public static final MethodHandle tiffProbe = h("cds_tiff_probe", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS));
     // the single-pair call behind a micro-batching queue with a device-side target cache (include/cdsgpu.h, cds_pairq_*)

@@ -1,5 +1,5 @@
 """One cds_ctx over all visible devices: dense / top-K / streaming searches (pixels and TIFF files, library from TIFF files, all
-matches) must equal the single-device results."""
+matches, best matches selected on the device) must equal the single-device results."""
 import sys, numpy as np
 sys.path.insert(0, ".")
 from colormipsearch_b200 import capi
@@ -16,6 +16,8 @@ pm = rng.integers(0, 6, 600); pt = rng.integers(0, NS, 600)
 has = (np.arange(NS) % 11 != 5).astype(np.uint8)
 pfiles = [capi.png_encode_gray16(g, -1 if i % 2 else 0) for i, g in enumerate(grads)]
 tfiles = [capi.tiff_encode_rgb(t, 8, 32773) for t in targets[:NS]]
+lines = ["R%dG%02d" % (10 + i // 7, i // 7) for i in range(200)]           # lines of 7 targets, samples of 2
+groups = capi.TargetGroups(lines, ["%d" % (i // 2) for i in range(200)])
 res = {}
 for nd in (1, 0):
     ctx = capi.Context(n_dev=nd)
@@ -39,6 +41,8 @@ for nd in (1, 0):
     qs, qmir, _ = q.drive(targets[:40], (np.arange(40) + 1).astype(np.uint64), qpm, qpt, 16)
     q.close()
     res[nd] = res[nd] + (shape_res, (qs, qmir, qpm, qpt))
+    res[nd] = res[nd] + ([(ms.search_best_matches(lib, groups, 1.0, *lim), ms.search_stream_best_matches_tiff(files, groups, 1.0, *lim))
+                          for lim in ((300, 1, 1), (5, 3, 2), (0, 0, 0))],)
     ms.close(); lib.close(); lib2.close(); ctx.close()
 a, b = res[1], res[0]
 print("dense equal:", np.array_equal(a[0][0], b[0][0]), np.array_equal(a[0][1], b[0][1]))
@@ -60,3 +64,6 @@ for name, i in (("shape pairs (pixels)", 2), ("shape pairs (TIFF)", 3), ("shape 
 for nd, r in ((1, a), (0, b)):
     qs, qmir, qpm, qpt = r[8]
     print("pair queue (devices %s) == dense:" % ("1" if nd else "all"), np.array_equal(qs, r[0][0][qpm, qpt]) and np.array_equal(qmir, r[0][1][qpm, qpt].astype(bool)))
+best_ok = all(all(np.array_equal(x, y) for x, y in zip(r1, r2)) for p1, p2 in zip(a[9], b[9]) for r1, r2 in zip(p1, p2))
+files_ok = all(all(np.array_equal(x, y) for x, y in zip(p[0], p[1])) for r in (a, b) for p in r[9])
+print("best matches (resident, TIFF files) single == multi:", best_ok, "; files == resident:", files_ok)
