@@ -478,7 +478,8 @@ cds_status cds_library::ensure_occupancy(int rings)
             }
             CDS_CUDA(ctx, e);
         }
-        launch_occupancy(sh.planes, g, sh.occ_done, nl - sh.occ_done, rings, bpitch, sh.valid, std::min<int64_t>(sh.cap_local, kValidChunk), sh.occ, ds.stream);
+        launch_occupancy(sh.planes, g, sh.occ_done, nl - sh.occ_done, rings, bpitch, sh.valid, std::min<int64_t>(sh.cap_local, kValidChunk), sh.occ, ds.stream,
+                         false, true);
         ctx->stats.kernel_launches += 2 * ((nl - sh.occ_done + kValidChunk - 1) / kValidChunk);
         CDS_CUDA(ctx, cudaGetLastError());
         sh.occ_done = nl;
@@ -1105,7 +1106,7 @@ cds_status launch_match_view(cds_ctx *ctx, const cds_maskset *ms, const TargetVi
     if (cand_ok) {
         int launches = launch_pixelmatch_cand(ms->d_descs[d] + m0, mc, tv.planes, tv.g, tv.n, tv.occ, tv.bpitch,
                                               ms->d_groups[d] + m0 / CDS_PALETTE_GROUP, ms->params.xy_shift, ms->params.mirror != 0,
-                                              d_scores, scratch, stream, ms->wide_lpal);
+                                              d_scores, scratch, stream, ms->wide_lpal, tv.bands);
         ctx->stats.kernel_launches += launches;
         ctx->stats.match_kernel_launches += launches;
         ctx->stats.match_kernel = 1;
@@ -1149,6 +1150,7 @@ cds_status launch_match(cds_ctx *ctx, const cds_maskset *ms, cds_library *lib, i
     tv.n = n_local;
     tv.occ_ready = lib->shards[d].occ && lib->shards[d].occ_done >= n_local && lib->occ_rings == ms->params.xy_shift / 2 &&
                    lib->occ_threshold == lib->baked_threshold;
+    tv.bands = tv.occ_ready;
     return launch_match_view(ctx, ms, tv, d, m0, mc, d_scores, ds.stream, ds.ev0, ds.ev1);
 }
 

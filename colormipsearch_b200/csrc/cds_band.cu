@@ -152,7 +152,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_band_kernel(cons
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int rowpitch = occupancy_row_pitch(p.bpitch);
-    const int any_off = CDS_NUM_SECTORS * p.bpitch;          // the OR over the sectors
+    const int any_off = occupancy_any_offset(p.bpitch);      // the OR over the sectors
     const int bits_words = (p.rows_per_band / 4) * rowpitch;       // rows_per_band is a multiple of the tile height
     const BandSmem<GROUP> L(p.stage_words, p.n_bands, NV, bits_words);
     uint32_t *s_stage = reinterpret_cast<uint32_t *>(smem_raw + L.stage_off) + kPrePad;

@@ -61,6 +61,7 @@ struct CandParams {
     int n_stages;                   // band stages in flight (2 .. kMaxStages)
     int wait_mode;                  // how a warp waits for a band: 0 polls try_wait, 1 try_wait with a suspend-time hint, 2 test_wait + nanosleep
     long long *trace;               // profiling aid (CDSGPU_CAND_TRACE): SM clock of CTA 0's first items, [item][band][32 warps][2] (+ producer in slot 31)
+    int band_filter;                // words whose rank-band nibble shares no band with the target tile's are dropped (CDSGPU_CAND_NOBAND=1: off)
 };
 constexpr int kTraceItems = 8;
 
@@ -211,7 +212,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
     constexpr int NCT = NCW * 32;                     // consumer threads
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int rowpitch = occupancy_row_pitch(p.bpitch);
+    const int rowpitch = occupancy_stage_pitch(p.bpitch);          // the staged part of a tile row: sector rows, non-empty bits, band nibbles
     const int bits_words = (p.rows_per_band / 4) * rowpitch;       // rows_per_band is a multiple of the tile height
     const int NSTG = p.n_stages;
     const CandSmem<GROUP> L(p.stage_words, NS, bits_words, NCW, NSTG);
@@ -295,15 +296,18 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
                     if (done) { mbar_arrive(bar); break; }
                     const uint32_t bytes = (uint32_t) ((y1 - y0 + 2 * S) * pitch) * 4u;
                     const uint32_t *src = p.planes + p.g.row_offset(t, 0) + (long long) (y0 - S) * pitch;   // guard rows cover y0 - S < 0
-                    const uint32_t bbytes = (uint32_t) (((y1 - y0 + 3) / 4) * rowpitch) * 4u;
-                    const uint32_t *bsrc = p.occ + ((size_t) t * occupancy_tile_rows(H) + y0 / 4) * rowpitch;
-                    mbar_expect_tx(bar, bytes + bbytes);
-                    if (HINT) {
-                        bulk_load_hint(smem_u32(s_stage + (size_t) stage * stage_stride), src, bytes, bar, pol_stream);
-                        bulk_load_hint(smem_u32(s_bits + (size_t) stage * bits_words), bsrc, bbytes, bar, pol_stream);
-                    } else {
-                        bulk_load(smem_u32(s_stage + (size_t) stage * stage_stride), src, bytes, bar);
-                        bulk_load(smem_u32(s_bits + (size_t) stage * bits_words), bsrc, bbytes, bar);
+                    // the occupancy tile rows without their OR rows (which this kernel never reads): one copy per tile row
+                    const int n_trows = (y1 - y0 + 3) / 4;
+                    const uint32_t rbytes = (uint32_t) rowpitch * 4u;
+                    const uint32_t *bsrc = p.occ + ((size_t) t * occupancy_tile_rows(H) + y0 / 4) * occupancy_row_pitch(p.bpitch);
+                    mbar_expect_tx(bar, bytes + (uint32_t) n_trows * rbytes);
+                    if (HINT) bulk_load_hint(smem_u32(s_stage + (size_t) stage * stage_stride), src, bytes, bar, pol_stream);
+                    else bulk_load(smem_u32(s_stage + (size_t) stage * stage_stride), src, bytes, bar);
+                    for (int r = 0; r < n_trows; r++) {
+                        const uint32_t dst = smem_u32(s_bits + (size_t) stage * bits_words + (size_t) r * rowpitch);
+                        const uint32_t *rsrc = bsrc + (size_t) r * occupancy_row_pitch(p.bpitch);
+                        if (HINT) bulk_load_hint(dst, rsrc, rbytes, bar, pol_stream);
+                        else bulk_load(dst, rsrc, rbytes, bar);
                     }
                 }
                 if (done) break;
@@ -452,10 +456,22 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
             const uint32_t band_lo = bi->band_lo;
             const uint32_t *bits_y0 = s_bits + (size_t) stage * bits_words - band_lo;          // indexed by the entries' absolute occupancy word index
             const uint32_t sec_words = (uint32_t) (CDS_NUM_SECTORS * p.bpitch);
-            const uint32_t nz_off = (uint32_t) ((CDS_NUM_SECTORS + 1) * p.bpitch);    // the non-empty bits of a tile row, behind its OR row
+            const uint32_t nz_off = (uint32_t) occupancy_nz_offset(p.bpitch);        // the non-empty bits of a tile row, behind its sector rows
             const uint4 idle = make_uint4(0u, band_lo, 0u, 0u);
             auto scan_one = [&](uint4 w) {
-                const uint32_t c = w.x & bits_y0[w.y];                  // mask pixels of this word that can match
+                const uint32_t occ_i = w.y & kWordOccMask;
+                uint32_t c = w.x & bits_y0[occ_i];                      // mask pixels of this word that can match
+                // Rank-band filter.  The tile's nibble holds the band of every target pixel that any shifted variant of any pixel of
+                // the tile can read in this sector, the entry's nibble every band that one of its pixels' intervals (in this sector)
+                // touches.  A pixel matches a target pixel only when that pixel's rank lies in its interval, and then both nibbles
+                // share that rank's band; disjoint nibbles therefore mean that no pixel of the word can match in any variant, and
+                // dropping the word changes no count.  The nibble of word i of tile row ty is nibble i - ty * rowpitch of the row's
+                // nibble words, i.e. nibble i + ty * 7 rowpitch + 8 * band offset counted from bits_y0.
+                if (c && p.band_filter) {
+                    const uint32_t nib = occ_i + (w.w & 255u) * (7u * (uint32_t) rowpitch) + 8u * (uint32_t) occupancy_band_offset(p.bpitch);
+                    const uint32_t tb = (uint32_t) reinterpret_cast<const uint8_t *>(bits_y0)[nib >> 1] >> ((nib & 1u) * 4u);
+                    if ((tb & (w.y >> kWordBandShift)) == 0u) c = 0u;
+                }
                 // words with candidates are compacted first, so that the bit expansion runs on (nearly) full warps: when the new ones
                 // do not fit behind the queued ones, those are expanded first
                 const unsigned has = __ballot_sync(0xffffffffu, c != 0);
@@ -610,7 +626,7 @@ CandConfig cand_config(int xy_shift, const PlaneGeom &g, int n_warps, int n_stag
         if (n_bands > kMaxBands) break;
         size_t stage_words = (size_t) (R + 2 * S) * g.pitch;
         if (stage_words >= (1u << kCandOffsetBits)) continue;       // candidates address the band with kCandOffsetBits bits (and a bulk copy stays below 1 MB)
-        CandSmem<GROUP> L((int) stage_words, NS, (R / 4) * occupancy_row_pitch(bpitch), n_warps, n_stages);
+        CandSmem<GROUP> L((int) stage_words, NS, (R / 4) * occupancy_stage_pitch(bpitch), n_warps, n_stages);
         if (L.total <= budget) {
             c.rows_per_band = R; c.n_bands = n_bands; c.stage_words = (int) stage_words; c.smem_bytes = L.total; c.ok = true;
             return c;
@@ -630,7 +646,7 @@ int env_int(const char *name, int dflt)
 template <int GROUP, int NCW>
 int launch_cfg(const MaskDesc *masks, int n_masks, const uint32_t *planes, PlaneGeom g, int64_t n_targets,
                const uint32_t *occ, int bpitch, const PaletteGroup *groups, int xy_shift, int32_t *scores,
-               const MatchScratch &scratch, cudaStream_t s, int dev, bool wide)
+               const MatchScratch &scratch, cudaStream_t s, int dev, bool wide, bool band_nibbles)
 {
     const int n_stages = std::max(2, std::min(kMaxStages, cand_tuning().stages));
     CandConfig c = cand_config<GROUP>(xy_shift, g, NCW, n_stages, cand_tuning().max_rows);
@@ -648,6 +664,7 @@ int launch_cfg(const MaskDesc *masks, int n_masks, const uint32_t *planes, Plane
     p.ticket_skip = no_skip ? 0 : 1;
     p.wait_mode = cand_tuning().wait_mode;
     p.n_stages = n_stages;
+    p.band_filter = band_nibbles && !env_int("CDSGPU_CAND_NOBAND", 0);   // read at every launch: tests compare both settings in one process
     const int hint = cand_tuning().l2_hint;
     static const char *trace_path = std::getenv("CDSGPU_CAND_TRACE");
     p.trace = nullptr;
@@ -694,13 +711,21 @@ int launch_cfg(const MaskDesc *masks, int n_masks, const uint32_t *planes, Plane
 constexpr int kRowTiles = 256;      // W <= 2048: tile columns per tile row
 constexpr int kLists = 2 * CDS_NUM_SECTORS;      // (orientation, sector) bitmaps per mask tile row
 
+// Rank bands (occupancy_rank_band) that an interval [lo, lo + len] (SR units) touches, as a nibble; 0 for an empty interval.
+__device__ __forceinline__ uint32_t interval_band_nibble(uint32_t lo, uint32_t len)
+{
+    if (lo == CDS_IV_EMPTY) return 0u;
+    const uint32_t r0 = lo % CDS_SECTOR_STRIDE, r1 = min(r0 + len, (uint32_t) CDS_NUM_RANKS - 1u);
+    return (2u << occupancy_rank_band(r1)) - (1u << occupancy_rank_band(r0));
+}
+
 // Scatters the records of one mask TILE ROW (4 image rows) into the (orientation, sector) tile bitmaps: pixel (x, y) is bit
 // (y % 4) * 8 + (x % 8) of tile word x / 8.  A mask pixel goes into the list of the sector of each of its non-empty rank
 // intervals: its own sector (interval 1) and, near a sector boundary, one neighbouring sector (interval 2).  `pix` (may be null)
-// receives, per (y % 4, x), the pixel's palette index | own sector << 11.
+// receives, per (y % 4, x), the pixel's palette index | own sector << 11 | band nibble of interval 1 << 16 | of interval 2 << 20.
 __device__ __forceinline__ void build_tile_row_lists(const MaskDesc &md, int ty, int W, int H, bool mirror,
                                                      const cds_class_interval *__restrict__ class_tab,
-                                                     uint32_t (*bm)[kRowTiles] /* [kLists] */, uint16_t *pix, uint32_t *pix_cls = nullptr)
+                                                     uint32_t (*bm)[kRowTiles] /* [kLists] */, uint32_t *pix, uint32_t *pix_cls = nullptr)
 {
     const int lane = threadIdx.x & 31;
     for (int k = lane; k < kLists * kRowTiles; k += 32) bm[0][k] = 0;
@@ -714,7 +739,8 @@ __device__ __forceinline__ void build_tile_row_lists(const MaskDesc &md, int ty,
         const int xm = W - 1 - x;
         const int s1 = (int) (cls / CDS_NUM_RANKS);
         const cds_class_interval iv = class_tab[cls];
-        if (pix) pix[yy * (kRowTiles * 8) + x] = (uint16_t) ((md.crec ? (__ldg(md.crec + i) >> 21) : 0u) | ((uint32_t) s1 << 11));
+        if (pix) pix[yy * (kRowTiles * 8) + x] = (md.crec ? (__ldg(md.crec + i) >> 21) : 0u) | ((uint32_t) s1 << 11) |
+                                                  (interval_band_nibble(iv.lo1, iv.len1) << 16) | (interval_band_nibble(iv.lo2, iv.len2) << 20);
         if (pix_cls) pix_cls[yy * (kRowTiles * 8) + x] = cls;
         const uint32_t bn = 1u << (yy * 8 + (x & 7)), bmr = 1u << (yy * 8 + (xm & 7));
         if (iv.lo1 != CDS_IV_EMPTY) {
@@ -790,8 +816,8 @@ __global__ void __launch_bounds__(32) words_fill_kernel(const MaskDesc *__restri
                                                         uint4 *__restrict__ words, uint16_t *__restrict__ lpal)
 {
     __shared__ uint32_t s_bm[kLists][kRowTiles];
-    // per (y % 4, x): palette index | own sector << 11, or (WIDE) the pixel's colour class
-    __shared__ typename std::conditional<WIDE, uint32_t, uint16_t>::type s_pix[4 * kRowTiles * 8];
+    // per (y % 4, x): palette index | own sector << 11 | the intervals' band nibbles << 16, << 20, or (WIDE) the pixel's colour class
+    __shared__ uint32_t s_pix[4 * kRowTiles * 8];
     const int lane = threadIdx.x;
     const int ty = blockIdx.x, HT = gridDim.x;
     const int m = first_mask + blockIdx.y;
@@ -822,9 +848,10 @@ __global__ void __launch_bounds__(32) words_fill_kernel(const MaskDesc *__restri
             if (wbits) {
                 const uint32_t pos = out_w + (uint32_t) __popc(bal & lt);
                 uint32_t lrec = out_b + incl - pc;
-                words[pos] = make_uint4(wbits, (uint32_t) (ty * occupancy_row_pitch(tp) + sec * tp + k), lrec,
-                                        (uint32_t) ty | ((uint32_t) k << kWordMetaColShift) | ((uint32_t) o << kWordMetaOrientBit) |
-                                            ((uint32_t) sec << kWordMetaSectorShift) | mtag);
+                const uint4 e = make_uint4(wbits, (uint32_t) (ty * occupancy_stage_pitch(tp) + sec * tp + k), lrec,
+                                           (uint32_t) ty | ((uint32_t) k << kWordMetaColShift) | ((uint32_t) o << kWordMetaOrientBit) |
+                                               ((uint32_t) sec << kWordMetaSectorShift) | mtag);
+                uint32_t nib = 0u;          // the word's rank-band nibble: OR over its pixels of the bands of their interval in this sector
                 // palette references of the word's pixels, in bit order: index | (interval 2 ? 0x8000 : 0)
                 while (wbits) {
                     const int bit = __ffs((int) wbits) - 1;
@@ -836,10 +863,14 @@ __global__ void __launch_bounds__(32) words_fill_kernel(const MaskDesc *__restri
                         const cds_class_interval iv = class_tab[pv];
                         const bool own = pv / CDS_NUM_RANKS == (uint32_t) sec;
                         reinterpret_cast<uint32_t *>(lpal)[lrec++] = pack_interval_word(own ? iv.lo1 : iv.lo2, own ? iv.len1 : iv.len2);
+                        nib |= interval_band_nibble(own ? iv.lo1 : iv.lo2, own ? iv.len1 : iv.len2);
                     } else {
-                        lpal[lrec++] = (uint16_t) ((pv & 0x7FFu) | (((pv >> 11) & 7u) != (uint32_t) sec ? 0x8000u : 0u));
+                        const bool own = ((pv >> 11) & 7u) == (uint32_t) sec;
+                        lpal[lrec++] = (uint16_t) ((pv & 0x7FFu) | (own ? 0u : 0x8000u));
+                        nib |= (pv >> (own ? 16 : 20)) & 0xFu;
                     }
                 }
+                words[pos] = make_uint4(e.x, e.y | (nib << kWordBandShift), e.z, e.w);
             }
             out_w += (uint32_t) __popc(bal);
             out_b += __shfl_sync(0xffffffffu, incl, 31);
@@ -859,7 +890,7 @@ __global__ void __launch_bounds__(256) words_bucket_count_kernel(const uint4 *__
     const int g = blockIdx.y;
     const uint32_t e0 = gstart[(size_t) g * (HT + 1)], e1 = gstart[(size_t) g * (HT + 1) + HT];
     for (uint32_t i = e0 + blockIdx.x * blockDim.x + threadIdx.x; i < e1; i += gridDim.x * blockDim.x)
-        atomicAdd(&counts[(size_t) g * n_buckets + words[i].y], 1u);
+        atomicAdd(&counts[(size_t) g * n_buckets + (words[i].y & kWordOccMask)], 1u);
 }
 
 // one CTA per group: counts -> first entry of every bucket (absolute index), in place
@@ -892,7 +923,7 @@ __global__ void __launch_bounds__(256) words_bucket_scatter_kernel(const uint4 *
     const uint32_t e0 = gstart[(size_t) g * (HT + 1)], e1 = gstart[(size_t) g * (HT + 1) + HT];
     for (uint32_t i = e0 + blockIdx.x * blockDim.x + threadIdx.x; i < e1; i += gridDim.x * blockDim.x) {
         const uint4 e = words[i];
-        const size_t b = (size_t) g * n_buckets + e.y;
+        const size_t b = (size_t) g * n_buckets + (e.y & kWordOccMask);
         sorted[first[b] + atomicAdd(&cursor[b], 1u)] = e;
     }
 }
@@ -902,7 +933,7 @@ __global__ void __launch_bounds__(256) words_tocc_kernel(const uint4 *__restrict
 {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n_tocc) return;
-    tocc[j] = n_entries ? words[min(j << 5, n_entries - 1u)].y : 0u;
+    tocc[j] = n_entries ? words[min(j << 5, n_entries - 1u)].y & kWordOccMask : 0u;
 }
 
 }  // namespace
@@ -944,6 +975,8 @@ bool cand_kernel_supported(int xy_shift, const PlaneGeom &g)
     if (!(xy_shift == 0 || xy_shift == 2 || xy_shift == 4)) return false;
     if (xy_shift > g.guard || xy_shift > g.pitch - g.W || xy_shift > kPrePad) return false;
     if (g.W > 2048 || g.H > 1024) return false;
+    // word-list entries carry the occupancy word index in 24 bits (their rank-band nibble above it)
+    if ((size_t) occupancy_tile_rows(g.H) * occupancy_stage_pitch(occupancy_tile_pitch(g.W)) > kWordOccMask) return false;
     return cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 16, 2, 0).ok;
 }
 
@@ -980,7 +1013,7 @@ void launch_words_fill(const MaskDesc *masks, int n_masks, int W, int H, bool mi
 
 int launch_pixelmatch_cand(const MaskDesc *masks, int n_masks, const uint32_t *planes, PlaneGeom g, int64_t n_targets,
                            const uint32_t *occ, int bpitch, const PaletteGroup *groups, int xy_shift, bool mirror,
-                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal)
+                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal, bool band_nibbles)
 {
     (void) mirror;      // the word lists already say which orientations exist
     if (n_masks == 0 || n_targets == 0) return 0;
@@ -997,7 +1030,7 @@ int launch_pixelmatch_cand(const MaskDesc *masks, int n_masks, const uint32_t *p
     if (warps >= 31 && !cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 31, n_stages, cand_tuning().max_rows).ok) warps = 28;
     if (warps >= 28 && !cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 28, n_stages, cand_tuning().max_rows).ok) warps = 24;
     if (warps >= 24 && !cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 24, n_stages, cand_tuning().max_rows).ok) warps = 16;
-#define CDS_CAND_LAUNCH(NCW) launch_cfg<CDS_PALETTE_GROUP, NCW>(masks, n_masks, planes, g, n_targets, occ, bpitch, groups, xy_shift, scores, scratch, s, dev, wide_lpal)
+#define CDS_CAND_LAUNCH(NCW) launch_cfg<CDS_PALETTE_GROUP, NCW>(masks, n_masks, planes, g, n_targets, occ, bpitch, groups, xy_shift, scores, scratch, s, dev, wide_lpal, band_nibbles)
     if (warps >= 31) return CDS_CAND_LAUNCH(31);
     if (warps >= 28) return CDS_CAND_LAUNCH(28);
     if (warps >= 24) return CDS_CAND_LAUNCH(24);

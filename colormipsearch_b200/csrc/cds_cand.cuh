@@ -16,7 +16,10 @@ namespace cds {
 // occupancy words --, then whatever) with a row-start table gstart[tile rows + 1], so the entries that concern a band of image rows are one contiguous
 // range that is cut into equal tickets regardless of mask boundaries.  One 16-byte entry per word:
 //     bits : the tile word
-//     occ  : index of the matching occupancy word inside a target's bitmaps: tile row * occupancy_row_pitch + sector * pitch + tile column
+//     occ  : bits 0..23: index of the matching occupancy word inside a target's bitmaps: tile row * occupancy_stage_pitch + sector * pitch
+//            + tile column (< 2^20 at W <= 2048, H <= 1024); bits 24..27: the word's rank-band nibble, the OR over its set bits of the
+//            rank bands (occupancy_rank_band) that the pixel's interval in this list's sector touches.  Readers mask the index with
+//            kWordOccMask.
 //     lrec : index into the group's `lpal` array of the palette reference of the word's LOWEST set bit; set bit b has
 //            lpal[lrec + popc(bits below b)] = palette index | 0x8000 when the pixel is in this list through its interval 2
 //            WIDE lists (a group of the set has more colour classes than a palette holds, e.g. brightness-scaled LM images used
@@ -31,6 +34,8 @@ constexpr int kWordMetaColShift = 8;
 constexpr int kWordMetaOrientBit = 16;
 constexpr int kWordMetaSectorShift = 17;
 constexpr int kWordMetaMaskShift = 22;
+constexpr uint32_t kWordOccMask = (1u << 24) - 1u;
+constexpr int kWordBandShift = 24;
 
 bool cand_kernel_supported(int xy_shift, const PlaneGeom &g);
 
@@ -60,7 +65,7 @@ void launch_words_fill(const MaskDesc *masks, int n_masks, int W, int H, bool mi
 // Reorders every tile row's entries by occupancy word (`occ`), i.e. by (sector, tile column): afterwards the entries that meet one
 // target tile are neighbours, and the kernel skips the tickets whose occupancy words are all empty.  `tables` = scratch of
 // 2 * n_groups * words_bucket_count(W, H) words; `sorted` receives the entries (same size as `words`, must not alias it).
-inline size_t words_bucket_count(int W, int H) { return (size_t) occupancy_tile_rows(H) * occupancy_row_pitch(occupancy_tile_pitch(W)); }
+inline size_t words_bucket_count(int W, int H) { return (size_t) occupancy_tile_rows(H) * occupancy_stage_pitch(occupancy_tile_pitch(W)); }
 void launch_words_bucket_sort(const uint4 *words, const uint32_t *gstart, int n_groups, int W, int H, uint32_t *tables, uint4 *sorted, cudaStream_t s);
 // PaletteGroup::tocc of the SORTED list: the occupancy word of every 32nd entry, words_tocc_count(n_entries) words.
 inline uint32_t words_tocc_count(uint32_t n_entries) { return n_entries / 32 + 2; }
@@ -70,7 +75,7 @@ void launch_words_tocc(const uint4 *words, uint32_t n_entries, uint32_t *tocc, c
 // (PaletteGroup::palette / words / gstart / lpal).
 int launch_pixelmatch_cand(const MaskDesc *masks, int n_masks, const uint32_t *planes, PlaneGeom g, int64_t n_targets,
                            const uint32_t *occ, int bpitch, const PaletteGroup *groups, int xy_shift, bool mirror,
-                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal = false);
+                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal = false, bool band_nibbles = false);
 
 }  // namespace cds
 #endif

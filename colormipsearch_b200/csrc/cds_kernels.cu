@@ -308,7 +308,7 @@ __global__ void __launch_bounds__(256) occupancy_kernel(const uint32_t *__restri
         const uint32_t *vimg = valid + (size_t) tl * H * vrow_words;
         uint32_t *trow = occ + ((size_t) (t0 + tl) * HT + ty) * rowpitch;
         uint4 *orow = reinterpret_cast<uint4 *>(trow) + k;
-        uint32_t *nz = trow + (CDS_NUM_SECTORS + 1) * tp;          // the row's non-empty bits: zero on entry (launch_occupancy_kernel clears them)
+        uint32_t *nz = trow + occupancy_nz_offset(tp);          // the row's non-empty bits: zero on entry (launch_occupancy_kernel clears them)
         uint32_t any[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
         for (int s = 0; s < CDS_NUM_SECTORS; s++) {
@@ -326,7 +326,7 @@ __global__ void __launch_bounds__(256) occupancy_kernel(const uint32_t *__restri
                 atomicOr(&nz[bit >> 5], nib << (bit & 31));
             }
         }
-        orow[(size_t) CDS_NUM_SECTORS * (tp / 4)] = strip_to_tiles(any);
+        reinterpret_cast<uint4 *>(trow + occupancy_any_offset(tp))[k] = strip_to_tiles(any);
     }
 }
 
@@ -409,11 +409,11 @@ __global__ void __launch_bounds__(kOccThreads) occupancy_ring1_kernel(const uint
                     atomicOr(&s_nz[bit >> 5], nib << (bit & 31));
                 }
             }
-            orow[(size_t) CDS_NUM_SECTORS * (tp / 4)] = strip_to_tiles(any);
+            reinterpret_cast<uint4 *>(trow + occupancy_any_offset(tp))[k] = strip_to_tiles(any);
         }
         __syncthreads();
         if (active && ty < HT) {
-            uint32_t *nz = occ + ((size_t) (t0 + tl) * HT + ty) * rowpitch + (CDS_NUM_SECTORS + 1) * tp;
+            uint32_t *nz = occ + ((size_t) (t0 + tl) * HT + ty) * rowpitch + occupancy_nz_offset(tp);
             for (int i = k; i < nzw; i += kc) nz[i] = s_nz[i];
         }
     }
@@ -440,20 +440,90 @@ static void launch_occupancy_kernel(const uint32_t *valid, int H, int vp, int tp
         return;
     }
     // the generic kernel ORs its non-empty bits into rows that start from zero: one strided clear
-    cudaMemset2DAsync(occ + (size_t) t0 * HT * rowpitch + (size_t) (CDS_NUM_SECTORS + 1) * tp, (size_t) rowpitch * sizeof(uint32_t), 0,
+    cudaMemset2DAsync(occ + (size_t) t0 * HT * rowpitch + (size_t) occupancy_nz_offset(tp), (size_t) rowpitch * sizeof(uint32_t), 0,
                       (size_t) occupancy_nz_words(tp) * sizeof(uint32_t), (size_t) n * HT, s);
     if (rings == 0) occupancy_kernel<0><<<148 * 8, 256, 0, s>>>(valid, H, vp, tp, t0, n, occ);
     else if (rings == 1) occupancy_kernel<1><<<148 * 8, 256, 0, s>>>(valid, H, vp, tp, t0, n, occ);
     else occupancy_kernel<2><<<148 * 8, 256, 0, s>>>(valid, H, vp, tp, t0, n, occ);
 }
 
+// Rank-band nibbles (cds_kernels.cuh).  One CTA per (target, tile row).  The per-sector valid bits that the occupancy kernels read say which
+// pixels of the rows [4 ty - S, 4 ty + 3 + S] count (in the image, above the baked threshold, of that sector; a few per cent of them), so
+// only those pixels' code words are read, for their ranks; their band bits (sector * 4 + band) are ORed per column in shared memory.
+// Then every tile ORs the columns [8 tx - S, 8 tx + 7 + S], and the nibbles leave as whole words.
+constexpr int kBandThreads = 256;
+constexpr int kBandPad = 4;                                // >= the largest xyShift
+
+__global__ void __launch_bounds__(kBandThreads) occupancy_bands_kernel(const uint32_t *__restrict__ valid /* chunk-relative */, int vp,
+                                                                       const uint32_t *__restrict__ planes, PlaneGeom g, int64_t t0, int S,
+                                                                       int tp, uint32_t *__restrict__ occ)
+{
+    extern __shared__ uint32_t s_col[];                    // [kBandPad + tp * 8 + kBandPad] column bits, then [tp] tile bits
+    const int ty = blockIdx.x, HT = gridDim.x;
+    const int64_t tl = blockIdx.y, t = t0 + tl;
+    const int ncol = tp * 8;
+    uint32_t *s_tile = s_col + ncol + 2 * kBandPad;
+    for (int i = threadIdx.x; i < ncol + 2 * kBandPad; i += kBandThreads) s_col[i] = 0u;
+    __syncthreads();
+    const int ya = max(4 * ty - S, 0), yb = min(4 * ty + 3 + S, g.H - 1);
+    const uint32_t *plane = planes + g.row_offset(t, 0);
+    const int n_words = (yb - ya + 1) * vp;
+    for (int i = threadIdx.x; i < n_words; i += kBandThreads) {
+        const int y = ya + i / vp, k = i % vp;
+        const uint32_t *vw = valid + ((size_t) tl * g.H + y) * CDS_NUM_SECTORS * vp + k;
+#pragma unroll
+        for (int sec = 0; sec < CDS_NUM_SECTORS; sec++) {
+            uint32_t m = __ldg(vw + sec * vp);
+            while (m) {
+                const int x = 32 * k + __ffs((int) m) - 1;
+                m &= m - 1u;
+                if (x >= g.W) break;
+                const uint32_t rank = (__ldg(plane + (size_t) y * g.pitch + x) >> CDS_CODE_SR_SHIFT) % CDS_SECTOR_STRIDE;
+                atomicOr(&s_col[x + kBandPad], 1u << (sec * 4 + (int) occupancy_rank_band(rank)));
+            }
+        }
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < tp; k += kBandThreads) {
+        uint32_t b = 0u;
+        for (int x = 8 * k - S; x <= 8 * k + 7 + S; x++) b |= s_col[x + kBandPad];
+        s_tile[k] = b;
+    }
+    __syncthreads();
+    uint32_t *out = occ + ((size_t) t * HT + ty) * occupancy_row_pitch(tp) + occupancy_band_offset(tp);
+    const int nbw = occupancy_band_words(tp);
+    for (int w = threadIdx.x; w < nbw; w += kBandThreads) {
+        uint32_t v = 0u;
+#pragma unroll
+        for (int j = 0; j < 8; j++) {
+            const int i = 8 * w + j;                       // sector tile word i = sector * tp + tile column
+            if (i < CDS_NUM_SECTORS * tp) v |= ((s_tile[i % tp] >> (4 * (i / tp))) & 0xFu) << (4 * j);
+        }
+        out[w] = v;
+    }
+}
+
+// targets [t0, t0 + n), whose valid bits are targets [0, n) of `valid`
+static void launch_occupancy_bands(const uint32_t *valid, const uint32_t *planes, PlaneGeom g, int64_t t0, int64_t n, int rings, int tp,
+                                   uint32_t *occ, cudaStream_t s)
+{
+    const size_t smem = (size_t) (tp * 8 + 2 * kBandPad + tp) * sizeof(uint32_t);
+    const int vp = occupancy_valid_pitch(g.W);
+    for (int64_t i0 = 0; i0 < n; i0 += 65535) {
+        const int64_t cnt = n - i0 < 65535 ? n - i0 : 65535;
+        occupancy_bands_kernel<<<dim3((unsigned) occupancy_tile_rows(g.H), (unsigned) cnt), kBandThreads, smem, s>>>(
+            valid + (size_t) i0 * g.H * CDS_NUM_SECTORS * vp, vp, planes, g, t0 + i0, 2 * rings, tp, occ);
+    }
+}
+
 void launch_occupancy(const uint32_t *planes, PlaneGeom g, int64_t t0, int64_t n, int rings, int tp,
-                      uint32_t *valid_scratch, int64_t scratch_targets, uint32_t *occ, cudaStream_t s, bool valid_ready)
+                      uint32_t *valid_scratch, int64_t scratch_targets, uint32_t *occ, cudaStream_t s, bool valid_ready, bool bands)
 {
     if (n == 0) return;
     const int vp = occupancy_valid_pitch(g.W);
     if (valid_ready) {      // the encoder already wrote the bits of targets [0, n) (launch_encode_rgb with `valid`)
         launch_occupancy_kernel(valid_scratch, g.H, vp, tp, t0, n, rings, occ, s);
+        if (bands) launch_occupancy_bands(valid_scratch, planes, g, t0, n, rings, tp, occ, s);
         return;
     }
     if (scratch_targets > 32768) scratch_targets = 32768;      // gridDim.y
@@ -462,6 +532,7 @@ void launch_occupancy(const uint32_t *planes, PlaneGeom g, int64_t t0, int64_t n
         dim3 grid(g.H, (unsigned) cnt);
         valid_bits_kernel<<<grid, 256, (size_t) CDS_NUM_SECTORS * vp * 4, s>>>(planes, g, t0 + i0, vp, valid_scratch);
         launch_occupancy_kernel(valid_scratch, g.H, vp, tp, t0 + i0, cnt, rings, occ, s);
+        if (bands) launch_occupancy_bands(valid_scratch, planes, g, t0 + i0, cnt, rings, tp, occ, s);
     }
 }
 

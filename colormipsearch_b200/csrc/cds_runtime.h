@@ -202,6 +202,7 @@ struct TargetView {
     int bpitch = 0;
     int64_t n = 0;                      // targets
     bool occ_ready = false;
+    bool bands = false;                 // the occupancy carries its rank-band nibbles (cds_kernels.cuh): the library's resident bitmaps only
 };
 // Picks and launches the match kernel for masks [m0, m0 + mc) of `ms` against `tv` on `stream`; ev0 / ev1 (may be null) are
 // recorded around it.  d_scores[(m - m0) * tv.n + t] = score word.
