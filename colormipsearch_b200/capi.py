@@ -159,6 +159,8 @@ SIGNATURES = {
     "cds_debug_pairq_drive": (C.c_int32, [_vp, _vp, C.c_int64, C.POINTER(C.c_uint64), _i32p, _i64p, C.c_int64, C.c_int32, _i32p, _u8p, _f64p]),
     "cds_debug_slice_numbers": (C.c_int32, [_vp, _vp, C.c_int64, _u16p]),
     "cds_debug_occupancy": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _vp]),
+    "cds_debug_library_bands": (C.c_int32, [_vp, C.c_int32, C.c_int32, _u8p]),
+    "cds_debug_cand_config": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i32p, _i32p, _i32p, _i64p]),
     "cds_debug_stream_plan": (C.c_int32, [C.c_int32, C.c_int64, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp]),
     "cds_debug_tiff_codes": (C.c_int32, [_vp, _vp, _i64p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _u32p, _u32p]),
 }
@@ -372,6 +374,14 @@ class Library:
 
     def __len__(self):
         return lib().cds_library_size(self.h)
+
+    def debug_bands(self, data_threshold, xy_shift):
+        """The rank-band bytes of the resident occupancy for these search parameters, uint8 [n][(H + 3) // 4][6 * tp]
+        (cds_debug_library_bands)."""
+        tp = ((self.W + 7) // 8 + 3) // 4 * 4
+        out = np.zeros((len(self), (self.H + 3) // 4, 6 * tp), np.uint8)
+        _check(lib().cds_debug_library_bands(self.h, int(data_threshold), int(xy_shift), out.ctypes.data_as(_u8p)), self.ctx.h)
+        return out
 
 
 class MaskSet:
@@ -809,6 +819,14 @@ def stream_plan(n_devices, n_targets, chunk, offsets=None, byte_cap=0xC0000000):
     _check(lib().cds_debug_stream_plan(int(n_devices), int(n_targets), int(chunk), None if off is None else off.ctypes.data_as(_vp), int(byte_cap), cap,
                                         dev.ctypes.data_as(_vp), first.ctypes.data_as(_vp), cnt.ctypes.data_as(_vp), C.byref(n)))
     return dev[:n.value], first[:n.value], cnt[:n.value]
+
+
+def cand_config(W, H, xy_shift, palette_entries, wide=False):
+    """cds_debug_cand_config: (warps, rows per band, stages, shared-memory bytes) of a candidate-kernel launch.  No device needed."""
+    warps, rows, stages, smem = C.c_int32(), C.c_int32(), C.c_int32(), C.c_int64()
+    _check(lib().cds_debug_cand_config(int(W), int(H), int(xy_shift), int(palette_entries), int(bool(wide)), C.byref(warps), C.byref(rows),
+                                       C.byref(stages), C.byref(smem)))
+    return warps.value, rows.value, stages.value, smem.value
 
 
 def tiff_decode_rgb_host(data, W, H):

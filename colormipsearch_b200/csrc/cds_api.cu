@@ -949,6 +949,7 @@ cds_status cds_maskset::sync_descs()
         if (d_words[d]) { ds.pool.free(d_words[d]); d_words[d] = nullptr; }
         if (d_wstart[d]) { ds.pool.free(d_wstart[d]); d_wstart[d] = nullptr; }
         std::vector<PaletteGroup> groups(std::max(n_groups, 1));
+        if (d == 0) n_pal.assign(n_groups, 0);
         for (auto &g : groups) { g.palette = nullptr; g.words = nullptr; g.gstart = nullptr; g.lpal = nullptr; g.tocc = nullptr; g.n_pal = 0; g.pad = 0; }
         if (compact_ok) {
             // palettes of the compact records: mark classes per group, number them, pack intervals, rewrite records
@@ -965,7 +966,7 @@ cds_status cds_maskset::sync_descs()
             if (st == CDS_OK) st = ctx->check(ds.pool.alloc((void **) &d_palettes[d], (size_t) n_groups * CDS_PALETTE_SIZE * sizeof(uint2)), "cudaMalloc(palettes)");
             if (st == CDS_OK) st = ctx->check(cudaMemcpyAsync(d_refs, refs.data(), refs.size() * sizeof(MaskClassRef), cudaMemcpyHostToDevice, ds.stream), "class refs H2D");
             if (st == CDS_OK) st = ctx->check(cudaMemsetAsync(d_flags, 0, slots * sizeof(uint32_t), ds.stream), "memset(palette flags)");
-            std::vector<int32_t> n_pal(n_groups, 0);
+            std::vector<int32_t> group_pal(n_groups, 0);
             if (st == CDS_OK) {
                 launch_palette_mark(d_refs, M, d_flags, ds.stream);
                 launch_palette_scan(d_flags, n_groups, d_pidx, d_npal, ds.stream);
@@ -974,7 +975,7 @@ cds_status cds_maskset::sync_descs()
                 ctx->stats.kernel_launches += 4;
                 st = ctx->check(cudaGetLastError(), "palette kernels");
             }
-            if (st == CDS_OK) st = ctx->check(cudaMemcpyAsync(n_pal.data(), d_npal, n_groups * sizeof(int32_t), cudaMemcpyDeviceToHost, ds.stream), "palette sizes D2H");
+            if (st == CDS_OK) st = ctx->check(cudaMemcpyAsync(group_pal.data(), d_npal, n_groups * sizeof(int32_t), cudaMemcpyDeviceToHost, ds.stream), "palette sizes D2H");
             if (st == CDS_OK) st = ctx->check(cudaStreamSynchronize(ds.stream), "palette build");
             ds.pool.free(d_refs);
             ds.pool.free(d_flags);
@@ -983,9 +984,10 @@ cds_status cds_maskset::sync_descs()
             if (st != CDS_OK) return st;
             int compact = 0;
             for (int g = 0; g < n_groups; g++) {
-                if (n_pal[g] >= CDS_PALETTE_SIZE) continue;   // the last palette index is reserved for idle lanes
+                if (group_pal[g] >= CDS_PALETTE_SIZE) continue;   // a staged palette keeps one entry for idle lanes
                 groups[g].palette = d_palettes[d] + (size_t) g * CDS_PALETTE_SIZE;
-                groups[g].n_pal = n_pal[g];
+                groups[g].n_pal = group_pal[g];
+                if (d == 0) n_pal[g] = group_pal[g];
                 compact++;
                 for (int m = g * CDS_PALETTE_GROUP; m < std::min(M, (g + 1) * CDS_PALETTE_GROUP); m++) h[m].crec = refs[m].crec;
             }
@@ -1104,9 +1106,12 @@ cds_status launch_match_view(cds_ctx *ctx, const cds_maskset *ms, const TargetVi
     const MatchScratch &scratch = ctx->devs[d].match_scratch;
     if (ev0) cudaEventRecord(ev0, stream);
     if (cand_ok) {
+        // the largest palette of the launch's groups, plus its idle entry: what the kernel stages
+        int pal_entries = 0;
+        for (int g = m0 / CDS_PALETTE_GROUP; g <= (m0 + mc - 1) / CDS_PALETTE_GROUP; g++) pal_entries = std::max(pal_entries, ms->n_pal[g] + 1);
         int launches = launch_pixelmatch_cand(ms->d_descs[d] + m0, mc, tv.planes, tv.g, tv.n, tv.occ, tv.bpitch,
                                               ms->d_groups[d] + m0 / CDS_PALETTE_GROUP, ms->params.xy_shift, ms->params.mirror != 0,
-                                              d_scores, scratch, stream, ms->wide_lpal, tv.bands);
+                                              d_scores, scratch, stream, ms->wide_lpal, tv.bands, pal_entries);
         ctx->stats.kernel_launches += launches;
         ctx->stats.match_kernel_launches += launches;
         ctx->stats.match_kernel = 1;
@@ -1133,6 +1138,54 @@ bool batched_kernel_supported(int xy_shift, const PlaneGeom &g)
     return cand_kernel_supported(xy_shift, g) || band_kernel_supported(xy_shift, g);
 }
 }  // namespace cds
+
+extern "C" cds_status cds_debug_cand_config(int32_t width, int32_t height, int32_t xy_shift, int32_t palette_entries, int32_t wide,
+                                            int32_t *warps, int32_t *rows_per_band, int32_t *stages, int64_t *smem_bytes)
+{
+    return cds::abi_guard("cds_debug_cand_config", [&]() -> cds_status {
+        if (width <= 0 || height <= 0 || width > 2048 || height > 1024 || !(xy_shift == 0 || xy_shift == 2 || xy_shift == 4) ||
+            palette_entries < 1 || palette_entries > CDS_PALETTE_SIZE || !warps || !rows_per_band || !stages || !smem_bytes) {
+            set_tls_error("cds_debug_cand_config: bad argument");
+            return CDS_ERR_BAD_ARG;
+        }
+        PlaneGeom g;
+        g.W = width; g.H = height; g.pitch = choose_pitch(width); g.guard = CDS_GUARD_ROWS;
+        const CandShape c = cand_launch_shape(xy_shift, g, wide ? 0 : palette_entries);
+        *warps = c.ok ? c.warps : 0;
+        *rows_per_band = c.ok ? c.rows_per_band : 0;
+        *stages = c.ok ? c.n_stages : 0;
+        *smem_bytes = c.ok ? (int64_t) c.smem_bytes : 0;
+        return CDS_OK;
+    });
+}
+
+extern "C" cds_status cds_debug_library_bands(cds_library *lib, int32_t data_threshold, int32_t xy_shift, uint8_t *bands_out)
+{
+    return cds::abi_guard("cds_debug_library_bands", [&]() -> cds_status {
+        if (!lib) { set_tls_error("cds_debug_library_bands: NULL library"); return CDS_ERR_BAD_ARG; }
+        cds_ctx *ctx = lib->ctx;
+        std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+        if (data_threshold < 0 || data_threshold > 255 || !(xy_shift == 0 || xy_shift == 2 || xy_shift == 4))
+            return ctx->fail(CDS_ERR_BAD_ARG, "cds_debug_library_bands: bad data_threshold or xy_shift");
+        if (lib->size == 0) return CDS_OK;
+        if (!bands_out) return ctx->fail(CDS_ERR_BAD_ARG, "cds_debug_library_bands: NULL output");
+        CDS_TRY(lib->bake(data_threshold));
+        CDS_TRY(lib->ensure_occupancy(xy_shift / 2));
+        if (lib->occ_on_the_fly) return ctx->fail(CDS_ERR_UNSUPPORTED, "cds_debug_library_bands: the library builds its occupancy per chunk");
+        const int tp = lib->bpitch, HT = occupancy_tile_rows(lib->g.H), row_bytes = CDS_NUM_SECTORS * tp;
+        for (int64_t gi = 0; gi < lib->size; gi++) {
+            int d = 0;
+            int64_t t = 0;
+            lib->locate(gi, d, t);
+            DevState &ds = ctx->devs[d];
+            CDS_CUDA(ctx, cudaSetDevice(ds.dev));
+            const uint32_t *src = lib->shards[d].occ + (size_t) t * occupancy_target_words(lib->g.W, lib->g.H) + occupancy_band_offset(tp);
+            CDS_CUDA(ctx, cudaMemcpy2D(bands_out + (size_t) gi * HT * row_bytes, (size_t) row_bytes, src, (size_t) occupancy_row_pitch(tp) * 4,
+                                       (size_t) row_bytes, (size_t) HT, cudaMemcpyDeviceToHost));
+        }
+        return CDS_OK;
+    });
+}
 
 namespace {
 

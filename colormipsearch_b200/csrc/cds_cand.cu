@@ -61,7 +61,8 @@ struct CandParams {
     int n_stages;                   // band stages in flight (2 .. kMaxStages)
     int wait_mode;                  // how a warp waits for a band: 0 polls try_wait, 1 try_wait with a suspend-time hint, 2 test_wait + nanosleep
     long long *trace;               // profiling aid (CDSGPU_CAND_TRACE): SM clock of CTA 0's first items, [item][band][32 warps][2] (+ producer in slot 31)
-    int band_filter;                // words whose rank-band nibble shares no band with the target tile's are dropped (CDSGPU_CAND_NOBAND=1: off)
+    int band_filter;                // words whose rank-band byte shares no band with the target tile's are dropped (CDSGPU_CAND_NOBAND=1: off)
+    int pal_entries;                // palette entries staged in shared memory (cand_staged_palette; 0 for WIDE lists), the last one idle
 };
 constexpr int kTraceItems = 8;
 
@@ -109,12 +110,12 @@ struct __align__(16) BandInfo {
 template <int GROUP>
 struct CandSmem {
     size_t stage_off, bits_off, pal_off, band_off, queue_off, wqueue_off, bar_off, next_off, item_off, sel_off, total;
-    __host__ __device__ CandSmem(int stage_words, int NS, int bits_words, int n_warps, int n_stages)
+    __host__ __device__ CandSmem(int stage_words, int NS, int bits_words, int n_warps, int n_stages, int pal_entries)
     {
         size_t o = 0;
         stage_off = o; o += (size_t) n_stages * (stage_words + kPrePad) * 4;
         bits_off = o;  o += (size_t) n_stages * bits_words * 4;
-        pal_off = o;   o += (size_t) CDS_PALETTE_SIZE * 8;
+        pal_off = o;   o += (size_t) pal_entries * 8;                               // a multiple of 16 entries: what follows stays 16-byte aligned
         wqueue_off = o; o += (size_t) n_warps * kWordQueue * 16;
         queue_off = o; o += (size_t) n_warps * kQueue * 8;
         bar_off = o;   o += 2 * kMaxStages * 8;
@@ -170,14 +171,14 @@ __device__ __forceinline__ uint32_t select_bit(uint32_t c, uint32_t r, const uin
 }
 
 // First half of an evaluation: the candidate's palette reference (palette index | 0x8000 for the second interval), an L2
-// access whose latency the caller hides behind the evaluation of the previous batch.
+// access whose latency the caller hides behind the evaluation of the previous batch.  Idle lanes get `idle`, the never-matching entry.
 // WIDE (groups with more colour classes than a shared-memory palette holds): lpal carries the packed interval itself, 32 bits per
 // set bit, and there is no palette.
 template <bool WIDE>
-__device__ __forceinline__ uint32_t fetch_palette_ref(uint2 cand, bool live, const uint16_t *__restrict__ lpal, uint64_t policy)
+__device__ __forceinline__ uint32_t fetch_palette_ref(uint2 cand, bool live, const uint16_t *__restrict__ lpal, uint64_t policy, uint32_t idle)
 {
     if (WIDE) return live ? __ldg(reinterpret_cast<const uint32_t *>(lpal) + cand.y) : CDS_PAL_EMPTY_LO;
-    uint32_t pr = CDS_PALETTE_SIZE - 1;                                         // the never-matching entry
+    uint32_t pr = idle;
     if (live) pr = policy ? ldg_hint_u16(lpal + cand.y, policy) : (uint32_t) __ldg(lpal + cand.y);
     return pr;
 }
@@ -189,7 +190,7 @@ __device__ __forceinline__ void eval_candidates(uint2 cand, uint32_t pr, const u
     constexpr int NS = Offsets<NRINGS>::N;
     uint32_t iv = pr;                                                           // WIDE: the reference IS the interval
     if (!WIDE) {
-        const uint2 pe = s_pal[pr & (CDS_PALETTE_SIZE - 1)];
+        const uint2 pe = s_pal[pr & 0x7FFFu];                                   // without the "interval 2" flag
         iv = (pr & 0x8000u) ? pe.y : pe.x;                                      // the interval that lives in this candidate's sector
     }
     const uint32_t lo = (iv & ((1u << CDS_PAL_LO_BITS) - 1)) << CDS_CODE_SR_SHIFT;
@@ -212,10 +213,10 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
     constexpr int NCT = NCW * 32;                     // consumer threads
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int rowpitch = occupancy_stage_pitch(p.bpitch);          // the staged part of a tile row: sector rows, non-empty bits, band nibbles
+    const int rowpitch = occupancy_stage_pitch(p.bpitch);          // the staged part of a tile row: sector rows, non-empty bits, band bytes
     const int bits_words = (p.rows_per_band / 4) * rowpitch;       // rows_per_band is a multiple of the tile height
     const int NSTG = p.n_stages;
-    const CandSmem<GROUP> L(p.stage_words, NS, bits_words, NCW, NSTG);
+    const CandSmem<GROUP> L(p.stage_words, NS, bits_words, NCW, NSTG, p.pal_entries);
     uint32_t *s_stage = reinterpret_cast<uint32_t *>(smem_raw + L.stage_off) + kPrePad;
     const int stage_stride = p.stage_words + kPrePad;
     const uint32_t *s_bits = reinterpret_cast<const uint32_t *>(smem_raw + L.bits_off);  // [stages][tile rows of a band * row pitch]
@@ -296,9 +297,10 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
                     if (done) { mbar_arrive(bar); break; }
                     const uint32_t bytes = (uint32_t) ((y1 - y0 + 2 * S) * pitch) * 4u;
                     const uint32_t *src = p.planes + p.g.row_offset(t, 0) + (long long) (y0 - S) * pitch;   // guard rows cover y0 - S < 0
-                    // the occupancy tile rows without their OR rows (which this kernel never reads): one copy per tile row
+                    // the occupancy tile rows without their OR rows (which this kernel never reads), and without their band bytes when
+                    // the filter is off (bitmaps built per chunk have none): one copy per tile row
                     const int n_trows = (y1 - y0 + 3) / 4;
-                    const uint32_t rbytes = (uint32_t) rowpitch * 4u;
+                    const uint32_t rbytes = (uint32_t) (p.band_filter ? rowpitch : occupancy_band_offset(p.bpitch)) * 4u;
                     const uint32_t *bsrc = p.occ + ((size_t) t * occupancy_tile_rows(H) + y0 / 4) * occupancy_row_pitch(p.bpitch);
                     mbar_expect_tx(bar, bytes + (uint32_t) n_trows * rbytes);
                     if (HINT) bulk_load_hint(smem_u32(s_stage + (size_t) stage * stage_stride), src, bytes, bar, pol_stream);
@@ -348,8 +350,10 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
             gwords = pg.words;
             glpal = pg.lpal;
             gtocc = pg.tocc;
-            if (!WIDE) for (int i = tid; i < pg.n_pal; i += NCT) s_pal[i] = pg.palette[i];
-            if (tid == 0) s_pal[CDS_PALETTE_SIZE - 1] = make_uint2(CDS_PAL_EMPTY_LO, CDS_PAL_EMPTY_LO);   // idle lanes point here
+            if (!WIDE) {
+                for (int i = tid; i < pg.n_pal; i += NCT) s_pal[i] = pg.palette[i];
+                if (tid == 0) s_pal[p.pal_entries - 1] = make_uint2(CDS_PAL_EMPTY_LO, CDS_PAL_EMPTY_LO);   // idle lanes point here
+            }
             consumer_barrier<NCT>();
             cur_gi = gi;
         }
@@ -376,7 +380,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
             bool pend = false;
             auto run_pending = [&]() { eval_candidates<NRINGS, WIDE>(pend_cand, pend_pr, band, pitch, s_pal, acc_base); };
             auto submit = [&](uint2 cand, bool live) {
-                const uint32_t pr = fetch_palette_ref<WIDE>(cand, live, glpal, pol_keep);
+                const uint32_t pr = fetch_palette_ref<WIDE>(cand, live, glpal, pol_keep, (uint32_t) p.pal_entries - 1u);
                 if (pend) run_pending();
                 pend_cand = cand; pend_pr = pr; pend = true;
             };
@@ -461,15 +465,15 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) pixelmatch_cand_kernel(cons
             auto scan_one = [&](uint4 w) {
                 const uint32_t occ_i = w.y & kWordOccMask;
                 uint32_t c = w.x & bits_y0[occ_i];                      // mask pixels of this word that can match
-                // Rank-band filter.  The tile's nibble holds the band of every target pixel that any shifted variant of any pixel of
-                // the tile can read in this sector, the entry's nibble every band that one of its pixels' intervals (in this sector)
-                // touches.  A pixel matches a target pixel only when that pixel's rank lies in its interval, and then both nibbles
-                // share that rank's band; disjoint nibbles therefore mean that no pixel of the word can match in any variant, and
-                // dropping the word changes no count.  The nibble of word i of tile row ty is nibble i - ty * rowpitch of the row's
-                // nibble words, i.e. nibble i + ty * 7 rowpitch + 8 * band offset counted from bits_y0.
+                // Rank-band filter.  The tile's byte holds the band of every target pixel that any shifted variant of any pixel of
+                // the tile can read in this sector, the entry's byte every band that one of its pixels' intervals (in this sector)
+                // touches.  A pixel matches a target pixel only when that pixel's rank lies in its interval, and then both bytes
+                // share that rank's band; disjoint bytes therefore mean that no pixel of the word can match in any variant, and
+                // dropping the word changes no count.  The byte of word i of tile row ty is byte i - ty * rowpitch of the row's
+                // band words, i.e. byte i + ty * 3 rowpitch + 4 * band offset counted from bits_y0.
                 if (c && p.band_filter) {
-                    const uint32_t nib = occ_i + (w.w & 255u) * (7u * (uint32_t) rowpitch) + 8u * (uint32_t) occupancy_band_offset(p.bpitch);
-                    const uint32_t tb = (uint32_t) reinterpret_cast<const uint8_t *>(bits_y0)[nib >> 1] >> ((nib & 1u) * 4u);
+                    const uint32_t bi = occ_i + (w.w & 255u) * (3u * (uint32_t) rowpitch) + 4u * (uint32_t) occupancy_band_offset(p.bpitch);
+                    const uint32_t tb = reinterpret_cast<const uint8_t *>(bits_y0)[bi];
                     if ((tb & (w.y >> kWordBandShift)) == 0u) c = 0u;
                 }
                 // words with candidates are compacted first, so that the bit expansion runs on (nearly) full warps: when the new ones
@@ -611,8 +615,9 @@ struct CandConfig {
     bool ok;
 };
 
+// `pal_entries`: palette entries staged (cand_staged_palette)
 template <int GROUP>
-CandConfig cand_config(int xy_shift, const PlaneGeom &g, int n_warps, int n_stages, int max_rows)
+CandConfig cand_config(int xy_shift, const PlaneGeom &g, int n_warps, int n_stages, int max_rows, int pal_entries)
 {
     const int bpitch = occupancy_tile_pitch(g.W);
     CandConfig c{};
@@ -626,7 +631,7 @@ CandConfig cand_config(int xy_shift, const PlaneGeom &g, int n_warps, int n_stag
         if (n_bands > kMaxBands) break;
         size_t stage_words = (size_t) (R + 2 * S) * g.pitch;
         if (stage_words >= (1u << kCandOffsetBits)) continue;       // candidates address the band with kCandOffsetBits bits (and a bulk copy stays below 1 MB)
-        CandSmem<GROUP> L((int) stage_words, NS, (R / 4) * occupancy_stage_pitch(bpitch), n_warps, n_stages);
+        CandSmem<GROUP> L((int) stage_words, NS, (R / 4) * occupancy_stage_pitch(bpitch), n_warps, n_stages, pal_entries);
         if (L.total <= budget) {
             c.rows_per_band = R; c.n_bands = n_bands; c.stage_words = (int) stage_words; c.smem_bytes = L.total; c.ok = true;
             return c;
@@ -646,10 +651,10 @@ int env_int(const char *name, int dflt)
 template <int GROUP, int NCW>
 int launch_cfg(const MaskDesc *masks, int n_masks, const uint32_t *planes, PlaneGeom g, int64_t n_targets,
                const uint32_t *occ, int bpitch, const PaletteGroup *groups, int xy_shift, int32_t *scores,
-               const MatchScratch &scratch, cudaStream_t s, int dev, bool wide, bool band_nibbles)
+               const MatchScratch &scratch, cudaStream_t s, int dev, bool wide, bool band_bytes, int pal_entries)
 {
     const int n_stages = std::max(2, std::min(kMaxStages, cand_tuning().stages));
-    CandConfig c = cand_config<GROUP>(xy_shift, g, NCW, n_stages, cand_tuning().max_rows);
+    CandConfig c = cand_config<GROUP>(xy_shift, g, NCW, n_stages, cand_tuning().max_rows, pal_entries);
     if (!c.ok) return 0;
     CandParams p;
     p.masks = masks; p.n_masks = n_masks; p.planes = planes; p.g = g; p.n_targets = n_targets; p.scores = scores;
@@ -664,7 +669,8 @@ int launch_cfg(const MaskDesc *masks, int n_masks, const uint32_t *planes, Plane
     p.ticket_skip = no_skip ? 0 : 1;
     p.wait_mode = cand_tuning().wait_mode;
     p.n_stages = n_stages;
-    p.band_filter = band_nibbles && !env_int("CDSGPU_CAND_NOBAND", 0);   // read at every launch: tests compare both settings in one process
+    p.band_filter = band_bytes && !env_int("CDSGPU_CAND_NOBAND", 0);   // read at every launch: tests compare both settings in one process
+    p.pal_entries = pal_entries;
     const int hint = cand_tuning().l2_hint;
     static const char *trace_path = std::getenv("CDSGPU_CAND_TRACE");
     p.trace = nullptr;
@@ -711,8 +717,8 @@ int launch_cfg(const MaskDesc *masks, int n_masks, const uint32_t *planes, Plane
 constexpr int kRowTiles = 256;      // W <= 2048: tile columns per tile row
 constexpr int kLists = 2 * CDS_NUM_SECTORS;      // (orientation, sector) bitmaps per mask tile row
 
-// Rank bands (occupancy_rank_band) that an interval [lo, lo + len] (SR units) touches, as a nibble; 0 for an empty interval.
-__device__ __forceinline__ uint32_t interval_band_nibble(uint32_t lo, uint32_t len)
+// Rank bands (occupancy_rank_band) that an interval [lo, lo + len] (SR units) touches, as a byte; 0 for an empty interval.
+__device__ __forceinline__ uint32_t interval_band_byte(uint32_t lo, uint32_t len)
 {
     if (lo == CDS_IV_EMPTY) return 0u;
     const uint32_t r0 = lo % CDS_SECTOR_STRIDE, r1 = min(r0 + len, (uint32_t) CDS_NUM_RANKS - 1u);
@@ -722,7 +728,7 @@ __device__ __forceinline__ uint32_t interval_band_nibble(uint32_t lo, uint32_t l
 // Scatters the records of one mask TILE ROW (4 image rows) into the (orientation, sector) tile bitmaps: pixel (x, y) is bit
 // (y % 4) * 8 + (x % 8) of tile word x / 8.  A mask pixel goes into the list of the sector of each of its non-empty rank
 // intervals: its own sector (interval 1) and, near a sector boundary, one neighbouring sector (interval 2).  `pix` (may be null)
-// receives, per (y % 4, x), the pixel's palette index | own sector << 11 | band nibble of interval 1 << 16 | of interval 2 << 20.
+// receives, per (y % 4, x), the pixel's palette index | own sector << 11 | band byte of interval 1 << 16 | of interval 2 << 24.
 __device__ __forceinline__ void build_tile_row_lists(const MaskDesc &md, int ty, int W, int H, bool mirror,
                                                      const cds_class_interval *__restrict__ class_tab,
                                                      uint32_t (*bm)[kRowTiles] /* [kLists] */, uint32_t *pix, uint32_t *pix_cls = nullptr)
@@ -740,7 +746,7 @@ __device__ __forceinline__ void build_tile_row_lists(const MaskDesc &md, int ty,
         const int s1 = (int) (cls / CDS_NUM_RANKS);
         const cds_class_interval iv = class_tab[cls];
         if (pix) pix[yy * (kRowTiles * 8) + x] = (md.crec ? (__ldg(md.crec + i) >> 21) : 0u) | ((uint32_t) s1 << 11) |
-                                                  (interval_band_nibble(iv.lo1, iv.len1) << 16) | (interval_band_nibble(iv.lo2, iv.len2) << 20);
+                                                  (interval_band_byte(iv.lo1, iv.len1) << 16) | (interval_band_byte(iv.lo2, iv.len2) << 24);
         if (pix_cls) pix_cls[yy * (kRowTiles * 8) + x] = cls;
         const uint32_t bn = 1u << (yy * 8 + (x & 7)), bmr = 1u << (yy * 8 + (xm & 7));
         if (iv.lo1 != CDS_IV_EMPTY) {
@@ -816,7 +822,7 @@ __global__ void __launch_bounds__(32) words_fill_kernel(const MaskDesc *__restri
                                                         uint4 *__restrict__ words, uint16_t *__restrict__ lpal)
 {
     __shared__ uint32_t s_bm[kLists][kRowTiles];
-    // per (y % 4, x): palette index | own sector << 11 | the intervals' band nibbles << 16, << 20, or (WIDE) the pixel's colour class
+    // per (y % 4, x): palette index | own sector << 11 | the intervals' band bytes << 16, << 24, or (WIDE) the pixel's colour class
     __shared__ uint32_t s_pix[4 * kRowTiles * 8];
     const int lane = threadIdx.x;
     const int ty = blockIdx.x, HT = gridDim.x;
@@ -851,7 +857,7 @@ __global__ void __launch_bounds__(32) words_fill_kernel(const MaskDesc *__restri
                 const uint4 e = make_uint4(wbits, (uint32_t) (ty * occupancy_stage_pitch(tp) + sec * tp + k), lrec,
                                            (uint32_t) ty | ((uint32_t) k << kWordMetaColShift) | ((uint32_t) o << kWordMetaOrientBit) |
                                                ((uint32_t) sec << kWordMetaSectorShift) | mtag);
-                uint32_t nib = 0u;          // the word's rank-band nibble: OR over its pixels of the bands of their interval in this sector
+                uint32_t bands = 0u;        // the word's rank-band byte: OR over its pixels of the bands of their interval in this sector
                 // palette references of the word's pixels, in bit order: index | (interval 2 ? 0x8000 : 0)
                 while (wbits) {
                     const int bit = __ffs((int) wbits) - 1;
@@ -863,14 +869,14 @@ __global__ void __launch_bounds__(32) words_fill_kernel(const MaskDesc *__restri
                         const cds_class_interval iv = class_tab[pv];
                         const bool own = pv / CDS_NUM_RANKS == (uint32_t) sec;
                         reinterpret_cast<uint32_t *>(lpal)[lrec++] = pack_interval_word(own ? iv.lo1 : iv.lo2, own ? iv.len1 : iv.len2);
-                        nib |= interval_band_nibble(own ? iv.lo1 : iv.lo2, own ? iv.len1 : iv.len2);
+                        bands |= interval_band_byte(own ? iv.lo1 : iv.lo2, own ? iv.len1 : iv.len2);
                     } else {
                         const bool own = ((pv >> 11) & 7u) == (uint32_t) sec;
                         lpal[lrec++] = (uint16_t) ((pv & 0x7FFu) | (own ? 0u : 0x8000u));
-                        nib |= (pv >> (own ? 16 : 20)) & 0xFu;
+                        bands |= (pv >> (own ? 16 : 24)) & 0xFFu;
                     }
                 }
-                words[pos] = make_uint4(e.x, e.y | (nib << kWordBandShift), e.z, e.w);
+                words[pos] = make_uint4(e.x, e.y | (bands << kWordBandShift), e.z, e.w);
             }
             out_w += (uint32_t) __popc(bal);
             out_b += __shfl_sync(0xffffffffu, incl, 31);
@@ -975,9 +981,9 @@ bool cand_kernel_supported(int xy_shift, const PlaneGeom &g)
     if (!(xy_shift == 0 || xy_shift == 2 || xy_shift == 4)) return false;
     if (xy_shift > g.guard || xy_shift > g.pitch - g.W || xy_shift > kPrePad) return false;
     if (g.W > 2048 || g.H > 1024) return false;
-    // word-list entries carry the occupancy word index in 24 bits (their rank-band nibble above it)
+    // word-list entries carry the occupancy word index in 24 bits (their rank-band byte above it)
     if ((size_t) occupancy_tile_rows(g.H) * occupancy_stage_pitch(occupancy_tile_pitch(g.W)) > kWordOccMask) return false;
-    return cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 16, 2, 0).ok;
+    return cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 16, 2, 0, CDS_PALETTE_SIZE).ok;      // whatever the palettes of a later launch
 }
 
 void launch_words_count(const MaskDesc *masks, int n_masks, int W, int H, bool mirror, const cds_class_interval *class_tab,
@@ -1011,9 +1017,25 @@ void launch_words_fill(const MaskDesc *masks, int n_masks, int W, int H, bool mi
     }
 }
 
+CandShape cand_launch_shape(int xy_shift, const PlaneGeom &g, int pal_entries)
+{
+    // tuning knob (default picked from profiles/): consumer warps per CTA.  More warps need more
+    // shared memory for their queues; when the band stages no longer fit (xyShift 4: 34 accumulators per mask) fewer are used.
+    const int n_stages = std::max(2, std::min(kMaxStages, cand_tuning().stages));
+    const int staged = cand_staged_palette(pal_entries);
+    auto fits = [&](int w) { return cand_config<CDS_PALETTE_GROUP>(xy_shift, g, w, n_stages, cand_tuning().max_rows, staged); };
+    int warps = cand_tuning().warps;
+    if (warps >= 31 && !fits(31).ok) warps = 28;
+    if (warps >= 28 && !fits(28).ok) warps = 24;
+    if (warps >= 24 && !fits(24).ok) warps = 16;
+    warps = warps >= 31 ? 31 : warps >= 28 ? 28 : warps >= 24 ? 24 : 16;
+    const CandConfig c = fits(warps);
+    return CandShape{warps, c.rows_per_band, n_stages, c.smem_bytes, c.ok};
+}
+
 int launch_pixelmatch_cand(const MaskDesc *masks, int n_masks, const uint32_t *planes, PlaneGeom g, int64_t n_targets,
                            const uint32_t *occ, int bpitch, const PaletteGroup *groups, int xy_shift, bool mirror,
-                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal, bool band_nibbles)
+                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal, bool band_bytes, int pal_entries)
 {
     (void) mirror;      // the word lists already say which orientations exist
     if (n_masks == 0 || n_targets == 0) return 0;
@@ -1023,14 +1045,10 @@ int launch_pixelmatch_cand(const MaskDesc *masks, int n_masks, const uint32_t *p
     if (!scratch.work_counter || !scratch.acc) return 0;
     cudaMemsetAsync(scratch.work_counter, 0, sizeof(unsigned long long), s);
     cudaMemsetAsync(scratch.acc, 0, kMatchAccBytes, s);
-    // tuning knob (default picked from profiles/): consumer warps per CTA.  More warps need more
-    // shared memory for their queues; when the band stages no longer fit (xyShift 4: 34 accumulators per mask) fewer are used.
-    int warps = cand_tuning().warps;
-    const int n_stages = std::max(2, std::min(kMaxStages, cand_tuning().stages));
-    if (warps >= 31 && !cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 31, n_stages, cand_tuning().max_rows).ok) warps = 28;
-    if (warps >= 28 && !cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 28, n_stages, cand_tuning().max_rows).ok) warps = 24;
-    if (warps >= 24 && !cand_config<CDS_PALETTE_GROUP>(xy_shift, g, 24, n_stages, cand_tuning().max_rows).ok) warps = 16;
-#define CDS_CAND_LAUNCH(NCW) launch_cfg<CDS_PALETTE_GROUP, NCW>(masks, n_masks, planes, g, n_targets, occ, bpitch, groups, xy_shift, scores, scratch, s, dev, wide_lpal, band_nibbles)
+    if (wide_lpal) pal_entries = 0;         // WIDE lists carry their intervals: no palette is staged
+    const int warps = cand_launch_shape(xy_shift, g, pal_entries).warps;
+    const int staged = cand_staged_palette(pal_entries);
+#define CDS_CAND_LAUNCH(NCW) launch_cfg<CDS_PALETTE_GROUP, NCW>(masks, n_masks, planes, g, n_targets, occ, bpitch, groups, xy_shift, scores, scratch, s, dev, wide_lpal, band_bytes, staged)
     if (warps >= 31) return CDS_CAND_LAUNCH(31);
     if (warps >= 28) return CDS_CAND_LAUNCH(28);
     if (warps >= 24) return CDS_CAND_LAUNCH(24);

@@ -4,6 +4,8 @@
 
 #include "cds_kernels.cuh"
 
+#include <algorithm>
+
 namespace cds {
 
 // WORD LISTS of a mask group (built once per mask set, per device).
@@ -17,7 +19,7 @@ namespace cds {
 // range that is cut into equal tickets regardless of mask boundaries.  One 16-byte entry per word:
 //     bits : the tile word
 //     occ  : bits 0..23: index of the matching occupancy word inside a target's bitmaps: tile row * occupancy_stage_pitch + sector * pitch
-//            + tile column (< 2^20 at W <= 2048, H <= 1024); bits 24..27: the word's rank-band nibble, the OR over its set bits of the
+//            + tile column (< 2^20 at W <= 2048, H <= 1024); bits 24..31: the word's rank-band byte, the OR over its set bits of the
 //            rank bands (occupancy_rank_band) that the pixel's interval in this list's sector touches.  Readers mask the index with
 //            kWordOccMask.
 //     lrec : index into the group's `lpal` array of the palette reference of the word's LOWEST set bit; set bit b has
@@ -38,6 +40,18 @@ constexpr uint32_t kWordOccMask = (1u << 24) - 1u;
 constexpr int kWordBandShift = 24;
 
 bool cand_kernel_supported(int xy_shift, const PlaneGeom &g);
+
+// Palette entries a launch stages in shared memory: `pal_entries` = the largest palette of the launch's groups plus the idle entry that
+// idle lanes read (0 for WIDE lists, which read no palette), rounded up to 16.  The idle entry is the last staged one.
+inline int cand_staged_palette(int pal_entries) { return pal_entries <= 0 ? 0 : std::min((pal_entries + 15) / 16 * 16, CDS_PALETTE_SIZE); }
+// What a launch at this geometry and palette size runs with: consumer warps, band height, stages in flight and dynamic shared memory
+// (ok = false: no configuration fits).  Host only; tests read it through cds_debug_cand_config.
+struct CandShape {
+    int warps, rows_per_band, n_stages;
+    size_t smem_bytes;
+    bool ok;
+};
+CandShape cand_launch_shape(int xy_shift, const PlaneGeom &g, int pal_entries);
 
 // Tuning knobs of the candidate kernel (process-wide; defaults from the environment, changed through cds_ctx_set_option
 // "cand_wait_mode" / "cand_l2_hint" / "cand_warps" so that one process can sweep them).
@@ -72,10 +86,11 @@ inline uint32_t words_tocc_count(uint32_t n_entries) { return n_entries / 32 + 2
 void launch_words_tocc(const uint4 *words, uint32_t n_entries, uint32_t *tocc, cudaStream_t s);
 
 // Same contract as launch_pixelmatch_band (cds_band.cuh); every group needs a palette and its word lists
-// (PaletteGroup::palette / words / gstart / lpal).
+// (PaletteGroup::palette / words / gstart / lpal).  `pal_entries`: the largest n_pal + 1 over the launch's groups (0 for WIDE lists).
+// `band_bytes`: the occupancy carries its rank-band bytes (cds_kernels.cuh), and the kernel filters words with them.
 int launch_pixelmatch_cand(const MaskDesc *masks, int n_masks, const uint32_t *planes, PlaneGeom g, int64_t n_targets,
                            const uint32_t *occ, int bpitch, const PaletteGroup *groups, int xy_shift, bool mirror,
-                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal = false, bool band_nibbles = false);
+                           int32_t *scores, const MatchScratch &scratch, cudaStream_t s, bool wide_lpal, bool band_bytes, int pal_entries);
 
 }  // namespace cds
 #endif

@@ -774,7 +774,7 @@ extern "C" cds_status cds_debug_occupancy(cds_ctx *ctx, const uint32_t *valid, i
         CDS_CUDA(ctx, cudaMemsetAsync(d_occ, 0xA5, occ_words * sizeof(uint32_t), ds.stream));      // every word must be written by the kernels
         launch_occupancy(nullptr, g, 0, n, xy_shift / 2, tp, d_valid, n, d_occ, ds.stream, true);
         CDS_CUDA(ctx, cudaGetLastError());
-        // the hook's layout (cdsgpu.h): sector rows, OR row, non-empty bits -- the rank-band nibbles need code planes and are left out
+        // the hook's layout (cdsgpu.h): sector rows, OR row, non-empty bits -- the rank-band bytes need code planes and are left out
         const int rowpitch = occupancy_row_pitch(tp), nzw = occupancy_nz_words(tp), out_pitch = (CDS_NUM_SECTORS + 1) * tp + nzw;
         const size_t rows = (size_t) n * occupancy_tile_rows(height);
         auto part = [&](int dst_col, int src_col, int words) {

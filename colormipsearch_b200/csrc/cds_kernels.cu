@@ -447,23 +447,24 @@ static void launch_occupancy_kernel(const uint32_t *valid, int H, int vp, int tp
     else occupancy_kernel<2><<<148 * 8, 256, 0, s>>>(valid, H, vp, tp, t0, n, occ);
 }
 
-// Rank-band nibbles (cds_kernels.cuh).  One CTA per (target, tile row).  The per-sector valid bits that the occupancy kernels read say which
+// Rank-band bytes (cds_kernels.cuh).  One CTA per (target, tile row).  The per-sector valid bits that the occupancy kernels read say which
 // pixels of the rows [4 ty - S, 4 ty + 3 + S] count (in the image, above the baked threshold, of that sector; a few per cent of them), so
-// only those pixels' code words are read, for their ranks; their band bits (sector * 4 + band) are ORed per column in shared memory.
-// Then every tile ORs the columns [8 tx - S, 8 tx + 7 + S], and the nibbles leave as whole words.
+// only those pixels' code words are read, for their ranks; their band bits (sector * 8 + band, 48 of them) are ORed per column in shared
+// memory.  Then every tile ORs the columns [8 tx - S, 8 tx + 7 + S], and the bytes leave as whole words.
 constexpr int kBandThreads = 256;
 constexpr int kBandPad = 4;                                // >= the largest xyShift
+static_assert(CDS_NUM_SECTORS * CDS_RANK_BANDS <= 64, "a column's band bits are one 64-bit word");
 
 __global__ void __launch_bounds__(kBandThreads) occupancy_bands_kernel(const uint32_t *__restrict__ valid /* chunk-relative */, int vp,
                                                                        const uint32_t *__restrict__ planes, PlaneGeom g, int64_t t0, int S,
                                                                        int tp, uint32_t *__restrict__ occ)
 {
-    extern __shared__ uint32_t s_col[];                    // [kBandPad + tp * 8 + kBandPad] column bits, then [tp] tile bits
+    extern __shared__ unsigned long long s_col[];          // [kBandPad + tp * 8 + kBandPad] column bits, then [tp] tile bits
     const int ty = blockIdx.x, HT = gridDim.x;
     const int64_t tl = blockIdx.y, t = t0 + tl;
     const int ncol = tp * 8;
-    uint32_t *s_tile = s_col + ncol + 2 * kBandPad;
-    for (int i = threadIdx.x; i < ncol + 2 * kBandPad; i += kBandThreads) s_col[i] = 0u;
+    unsigned long long *s_tile = s_col + ncol + 2 * kBandPad;
+    for (int i = threadIdx.x; i < ncol + 2 * kBandPad; i += kBandThreads) s_col[i] = 0ull;
     __syncthreads();
     const int ya = max(4 * ty - S, 0), yb = min(4 * ty + 3 + S, g.H - 1);
     const uint32_t *plane = planes + g.row_offset(t, 0);
@@ -479,13 +480,13 @@ __global__ void __launch_bounds__(kBandThreads) occupancy_bands_kernel(const uin
                 m &= m - 1u;
                 if (x >= g.W) break;
                 const uint32_t rank = (__ldg(plane + (size_t) y * g.pitch + x) >> CDS_CODE_SR_SHIFT) % CDS_SECTOR_STRIDE;
-                atomicOr(&s_col[x + kBandPad], 1u << (sec * 4 + (int) occupancy_rank_band(rank)));
+                atomicOr(&s_col[x + kBandPad], 1ull << (sec * CDS_RANK_BANDS + (int) occupancy_rank_band(rank)));
             }
         }
     }
     __syncthreads();
     for (int k = threadIdx.x; k < tp; k += kBandThreads) {
-        uint32_t b = 0u;
+        unsigned long long b = 0ull;
         for (int x = 8 * k - S; x <= 8 * k + 7 + S; x++) b |= s_col[x + kBandPad];
         s_tile[k] = b;
     }
@@ -495,9 +496,9 @@ __global__ void __launch_bounds__(kBandThreads) occupancy_bands_kernel(const uin
     for (int w = threadIdx.x; w < nbw; w += kBandThreads) {
         uint32_t v = 0u;
 #pragma unroll
-        for (int j = 0; j < 8; j++) {
-            const int i = 8 * w + j;                       // sector tile word i = sector * tp + tile column
-            if (i < CDS_NUM_SECTORS * tp) v |= ((s_tile[i % tp] >> (4 * (i / tp))) & 0xFu) << (4 * j);
+        for (int j = 0; j < 4; j++) {
+            const int i = 4 * w + j;                       // sector tile word i = sector * tp + tile column
+            if (i < CDS_NUM_SECTORS * tp) v |= (uint32_t) ((s_tile[i % tp] >> (CDS_RANK_BANDS * (i / tp))) & 0xFFull) << (8 * j);
         }
         out[w] = v;
     }
@@ -507,7 +508,7 @@ __global__ void __launch_bounds__(kBandThreads) occupancy_bands_kernel(const uin
 static void launch_occupancy_bands(const uint32_t *valid, const uint32_t *planes, PlaneGeom g, int64_t t0, int64_t n, int rings, int tp,
                                    uint32_t *occ, cudaStream_t s)
 {
-    const size_t smem = (size_t) (tp * 8 + 2 * kBandPad + tp) * sizeof(uint32_t);
+    const size_t smem = (size_t) (tp * 8 + 2 * kBandPad + tp) * sizeof(unsigned long long);
     const int vp = occupancy_valid_pitch(g.W);
     for (int64_t i0 = 0; i0 < n; i0 += 65535) {
         const int64_t cnt = n - i0 < 65535 ? n - i0 : 65535;

@@ -87,32 +87,32 @@ __host__ __device__ inline int occupancy_valid_pitch(int W) { return (((W + 31) 
 __host__ __device__ inline int occupancy_tile_pitch(int W) { return (((W + 7) / 8) + 3) / 4 * 4; }
 __host__ __device__ inline int occupancy_tile_rows(int H) { return (H + 3) / 4; }
 // A tile row is laid out as
-//   [sector rows: CDS_NUM_SECTORS * tp words][non-empty bits: occupancy_nz_words(tp)][rank-band nibbles: occupancy_band_words(tp)][OR row: tp]
+//   [sector rows: CDS_NUM_SECTORS * tp words][non-empty bits: occupancy_nz_words(tp)][rank-band bytes: occupancy_band_words(tp)][OR row: tp]
 // The first three parts (occupancy_stage_pitch(tp) words) are what the candidate kernel stages per tile row; the word lists index
 // them (tile row * occupancy_stage_pitch + sector * tp + tile column).  The OR row, read by the band kernel only, comes last.
 //   * non-empty bits: one BIT per sector tile word, "this word is not empty" (bit i = word i of the tile row, i < CDS_NUM_SECTORS * tp).
 //     The candidate kernel's ticket tests read these.
-//   * rank-band nibbles: nibble i (bits 4 (i % 8) .. 4 (i % 8) + 3 of word i / 8) belongs to sector tile word i and has bit b set when
+//   * rank-band bytes: byte i (bits 8 (i % 4) .. 8 (i % 4) + 7 of word i / 4) belongs to sector tile word i and has bit b set when
 //     one of the target pixels that can set that word's bits has rank band b (occupancy_rank_band): a pixel of the word's sector,
 //     inside the image, above the baked threshold, in the rectangle [8 tx - S, 8 tx + 7 + S] x [4 ty - S, 4 ty + 3 + S] (S = xyShift).
 //     That rectangle is exactly the union of the shifted tile for xyShift 2 and 4 except in a last tile row that holds a single image
 //     row, where it is a superset; for xyShift 0 it is the tile itself.  Written by launch_occupancy with `bands` -- for the library's resident
-//     bitmaps, which serve every later search.  Bitmaps built per streamed chunk serve one search: there the nibbles cost more time than
+//     bitmaps, which serve every later search.  Bitmaps built per streamed chunk serve one search: there the bytes cost more time than
 //     the filter saves (DESIGN.md §4.1, v21), so they are not built and the candidate kernel runs without the filter.
 __host__ __device__ inline int occupancy_nz_words(int tp) { return ((CDS_NUM_SECTORS * tp + 31) / 32 + 3) / 4 * 4; }
-__host__ __device__ inline int occupancy_band_words(int tp) { return ((CDS_NUM_SECTORS * tp + 7) / 8 + 3) / 4 * 4; }
+__host__ __device__ inline int occupancy_band_words(int tp) { return ((CDS_NUM_SECTORS * tp + 3) / 4 + 3) / 4 * 4; }
 __host__ __device__ inline int occupancy_nz_offset(int tp) { return CDS_NUM_SECTORS * tp; }
 __host__ __device__ inline int occupancy_band_offset(int tp) { return CDS_NUM_SECTORS * tp + occupancy_nz_words(tp); }
 __host__ __device__ inline int occupancy_stage_pitch(int tp) { return occupancy_band_offset(tp) + occupancy_band_words(tp); }
 __host__ __device__ inline int occupancy_any_offset(int tp) { return occupancy_stage_pitch(tp); }
 __host__ __device__ inline int occupancy_row_pitch(int tp) { return occupancy_stage_pitch(tp) + tp; }
 __host__ __device__ inline size_t occupancy_target_words(int W, int H) { return (size_t) occupancy_tile_rows(H) * occupancy_row_pitch(occupancy_tile_pitch(W)); }
-// Rank bands: every sector's CDS_NUM_RANKS ranks cut into CDS_RANK_BANDS equal runs.  A fixed table, so that target nibbles and the
-// mask entries' nibbles (cds_cand.cu) agree without any data-dependent state.
-#define CDS_RANK_BANDS 4
+// Rank bands: every sector's CDS_NUM_RANKS ranks cut into CDS_RANK_BANDS equal runs.  A fixed table, so that the target tiles' bytes and
+// the mask entries' bytes (cds_cand.cu) agree without any data-dependent state.  One bit per band: at most 8.
+#define CDS_RANK_BANDS 8
 __host__ __device__ inline uint32_t occupancy_rank_band(uint32_t rank) { return rank * CDS_RANK_BANDS / CDS_NUM_RANKS; }
 int &occupancy_kernel_version();      // cds_ctx_set_option("occupancy_kernel")
-// `bands`: also the rank-band nibbles (from the valid bits and the ranks in the code planes, which must then be given).
+// `bands`: also the rank-band bytes (from the valid bits and the ranks in the code planes, which must then be given).
 void launch_occupancy(const uint32_t *planes, PlaneGeom g, int64_t t0, int64_t n, int rings, int tp,
                       uint32_t *valid_scratch, int64_t scratch_targets, uint32_t *occ, cudaStream_t s, bool valid_ready = false,
                       bool bands = false);

@@ -448,26 +448,29 @@ extern "C" cds_status cds_pairq_score(cds_pairq *q, int32_t mask_index, uint64_t
         bool pushed = false;                 // a resident target: the request is queued inside the lookup's critical section
         {
             std::unique_lock<std::mutex> lk(pd.mu);
-            auto it = anonymous ? pd.by_key.end() : pd.by_key.find(target_key);
-            if (it != pd.by_key.end()) {
-                req.slot = it->second;
-                CacheSlot &cs = pd.slots[req.slot];
-                cs.refs++;                                   // pins the slot while we wait for another caller's upload of the same image
-                pd.cv_slot.wait(lk, [&] { return !cs.loading; });
-                cs.refs--;
-                if (!cs.valid) { set_tls_error("cds_pairq_score: the upload of this target failed in another thread"); return CDS_ERR_CUDA; }
-                if (cs.ready_pending) req.ready = cs.ready;
-            } else {
-                // a free slot (least recently used, not referenced by a request in flight) and an upload lane
-                for (;;) {
-                    int victim = -1;
-                    for (int s : pd.lru) if (pd.slots[s].refs == 0) { victim = s; break; }
-                    if (victim >= 0) {
-                        for (size_t l = 0; l < pd.lanes.size(); l++) if (!pd.lanes[l].busy) { lane = (int) l; break; }
-                        if (lane >= 0) { req.slot = victim; break; }
-                    }
-                    pd.cv_slot.wait(lk);
+            for (;;) {
+                auto it = anonymous ? pd.by_key.end() : pd.by_key.find(target_key);
+                if (it != pd.by_key.end()) {
+                    req.slot = it->second;
+                    CacheSlot &cs = pd.slots[req.slot];
+                    cs.refs++;                                   // pins the slot while we wait for another caller's upload of the same image
+                    pd.cv_slot.wait(lk, [&] { return !cs.loading; });
+                    cs.refs--;
+                    if (!cs.valid) { set_tls_error("cds_pairq_score: the upload of this target failed in another thread"); return CDS_ERR_CUDA; }
+                    if (cs.ready_pending) req.ready = cs.ready;
+                    break;
                 }
+                // a free slot (least recently used, not referenced by a request in flight) and an upload lane
+                int victim = -1;
+                for (int s : pd.lru) if (pd.slots[s].refs == 0) { victim = s; break; }
+                if (victim >= 0) {
+                    for (size_t l = 0; l < pd.lanes.size(); l++) if (!pd.lanes[l].busy) { lane = (int) l; break; }
+                    if (lane >= 0) { req.slot = victim; break; }
+                }
+                // none yet: wait, then look the key up again -- another caller may have started uploading this image meanwhile
+                pd.cv_slot.wait(lk);
+            }
+            if (lane >= 0) {
                 CacheSlot &cs = pd.slots[req.slot];
                 auto old = pd.by_key.find(cs.key);
                 if (old != pd.by_key.end() && old->second == req.slot) pd.by_key.erase(old);

@@ -186,6 +186,7 @@ struct cds_maskset {
     std::vector<uint32_t *> d_words;                   // per device, word-list entries of all groups followed by their palette references (cds_cand.cuh)
     std::vector<uint32_t *> d_wstart;                  // per device, per-mask offsets and per-group row starts of the word lists
     int n_compact_groups = 0;                          // groups whose colour classes fit a shared-memory palette
+    std::vector<int32_t> n_pal;                        // per group, its palette's size (0 without a palette); the same on every device
     bool wide_lpal = false;                            // the word lists carry intervals instead of palette references (cds_cand.cuh: WIDE)
     bool words_built = false;                          // the candidate kernel's word lists exist on every device
     bool descs_dirty = true;
@@ -202,7 +203,7 @@ struct TargetView {
     int bpitch = 0;
     int64_t n = 0;                      // targets
     bool occ_ready = false;
-    bool bands = false;                 // the occupancy carries its rank-band nibbles (cds_kernels.cuh): the library's resident bitmaps only
+    bool bands = false;                 // the occupancy carries its rank-band bytes (cds_kernels.cuh): the library's resident bitmaps only
 };
 // Picks and launches the match kernel for masks [m0, m0 + mc) of `ms` against `tv` on `stream`; ev0 / ev1 (may be null) are
 // recorded around it.  d_scores[(m - m0) * tv.n + t] = score word.

@@ -520,6 +520,18 @@ cds_status cds_debug_tiff_codes(cds_ctx *ctx, const uint8_t *blob, const int64_t
  * 4): six sector rows of 8 x 4 tile words, their OR row, one "non-empty" bit per sector tile word.  The words between the rows are all written. */
 cds_status cds_debug_occupancy(cds_ctx *ctx, const uint32_t *valid, int64_t n, int32_t width, int32_t height, int32_t xy_shift,
                                uint32_t *occ_out);
+/* Test hook: the rank-band bytes that a search with data_threshold and xy_shift (0, 2, 4) finds in the library's resident occupancy
+ * (baking the library at data_threshold and building the occupancy first, as such a search does): uint8[size][(height + 3) / 4][6 * tp],
+ * tp as above; byte [t][ty][sector * tp + tx] has bit b set when a pixel of target t in that colour sector, inside the image, above
+ * data_threshold and in [8 tx - S, 8 tx + 7 + S] x [4 ty - S, 4 ty + 3 + S] (S = xy_shift) has rank band b = rank * 8 / 19820.
+ * CDS_ERR_UNSUPPORTED when the library has no room for resident occupancy and builds it per chunk. */
+cds_status cds_debug_library_bands(cds_library *lib, int32_t data_threshold, int32_t xy_shift, uint8_t *bands_out);
+/* Test hook (no device needed): how the candidate kernel would run at this image size, xy_shift (0, 2, 4) and palette size
+ * (palette_entries = the largest palette of the launch's mask groups plus one idle entry, 1..2048; ignored when wide != 0, since wide
+ * word lists read no palette): consumer warps per block, image rows per band, band stages in flight and dynamic shared memory in bytes.
+ * All four are 0 when no configuration fits. */
+cds_status cds_debug_cand_config(int32_t width, int32_t height, int32_t xy_shift, int32_t palette_entries, int32_t wide,
+                                 int32_t *warps, int32_t *rows_per_band, int32_t *stages, int64_t *smem_bytes);
 /* Test hook (no device needed): the chunk plan of the streaming searches over host targets -- entry i = (device, first target, count).
  * offsets == NULL: pixels (equal chunks of `chunk` targets, round-robin over the devices); otherwise the files' offsets [n_targets + 1]:
  * the first chunks of every device are 256, 512, ... files, what is left after the ramp is cut into equal chunks of at most `chunk`, and a
