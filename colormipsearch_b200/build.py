@@ -14,7 +14,7 @@ LIBDIR = os.path.join(HERE, "lib")
 SO = os.path.join(LIBDIR, "libcdsgpu.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-CU_SOURCES = ["cds_api.cu", "cds_stream.cu", "cds_kernels.cu", "cds_band.cu", "cds_cand.cu", "cds_topk.cu", "cds_synth.cu", "cds_shape.cu", "cds_ingest.cu", "cds_pairq.cu", "cds_inflate.cu", "cds_bestsel.cu"]
+CU_SOURCES = ["cds_api.cu", "cds_stream.cu", "cds_kernels.cu", "cds_band.cu", "cds_cand.cu", "cds_topk.cu", "cds_synth.cu", "cds_shape.cu", "cds_ingest.cu", "cds_pairq.cu", "cds_shape_pairq.cu", "cds_inflate.cu", "cds_bestsel.cu"]
 CPP_SOURCES = ["cds_tables.cpp", "cds_select.cpp", "cds_tiff.cpp", "cds_formats.cpp"]
 
 NVCC_FLAGS = [

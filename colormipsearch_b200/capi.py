@@ -157,6 +157,12 @@ SIGNATURES = {
     "cds_pairq_score": (C.c_int32, [_vp, C.c_int32, C.c_uint64, _vp, C.c_int32, C.c_int32, _i32p, _f64p, _i32p]),
     "cds_pairq_get_stats": (C.c_int32, [_vp, _i64p, _i64p, _i64p]),
     "cds_debug_pairq_drive": (C.c_int32, [_vp, _vp, C.c_int64, C.POINTER(C.c_uint64), _i32p, _i64p, C.c_int64, C.c_int32, _i32p, _u8p, _f64p]),
+    "cds_shape_pairq_create": (C.c_int32, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.POINTER(_vp)]),
+    "cds_shape_pairq_destroy": (None, [_vp]),
+    "cds_shape_pairq_score": (C.c_int32, [_vp, C.c_int32, C.c_uint64, _vp, _vp, _vp, C.c_int32, C.c_int32, _i64p, _i64p, _i32p]),
+    "cds_shape_pairq_get_stats": (C.c_int32, [_vp, _i64p, _i64p, _i64p]),
+    "cds_debug_shape_pairq_drive": (C.c_int32, [_vp, _vp, _vp, _vp, C.c_int64, C.POINTER(C.c_uint64), _i32p, _i64p, C.c_int64, C.c_int32,
+                                                _i64p, _i64p, _u8p, _f64p]),
     "cds_debug_slice_numbers": (C.c_int32, [_vp, _vp, C.c_int64, _u16p]),
     "cds_debug_occupancy": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _vp]),
     "cds_debug_library_bands": (C.c_int32, [_vp, C.c_int32, C.c_int32, _u8p]),
@@ -741,6 +747,61 @@ class ShapeMaskSet:
                                                 pair_target.ctypes.data_as(_i64p), n, gap.ctypes.data_as(_i64p), he.ctypes.data_as(_i64p),
                                                 mir.ctypes.data_as(_u8p)), self.ctx.h)
         return gap, he, mir.astype(bool)
+
+
+class ShapePairQueue:
+    """cds_shape_pairq_*: the shape score's single-pair call (Shape2DMatch...calculateMatchingScore) behind a micro-batching queue with a
+    device-side cache of derived target planes.  score() blocks and may be called from many threads."""
+
+    def __init__(self, ctx, shape_maskset, max_batch=64, max_wait_us=50, cache_targets=256):
+        self.ctx, self.sms = ctx, shape_maskset
+        h = _vp()
+        _check(lib().cds_shape_pairq_create(ctx.h, shape_maskset.h, int(max_batch), int(max_wait_us), int(cache_targets), C.byref(h)), ctx.h)
+        self.h = h
+        ctx._children.add(self)
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().cds_shape_pairq_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def score(self, mask_index, target_rgb, gradient, zgap_rgb=None, key=0):
+        """-> (gradient area gap, high expression area, mirrored); gradient None = missing supplier: (-1, -1, False)"""
+        target_rgb = None if target_rgb is None else np.ascontiguousarray(target_rgb, dtype=np.uint8)
+        gradient = None if gradient is None else np.ascontiguousarray(gradient, dtype=np.uint16)
+        zgap_rgb = None if zgap_rgb is None else np.ascontiguousarray(zgap_rgb, dtype=np.uint8)
+        H, W = (target_rgb.shape[0], target_rgb.shape[1]) if target_rgb is not None else (self.sms.H, self.sms.W)
+        g, he, m = C.c_int64(), C.c_int64(), C.c_int32()
+        _check(lib().cds_shape_pairq_score(self.h, int(mask_index), int(key), _ptr(target_rgb), _ptr(gradient), _ptr(zgap_rgb), W, H,
+                                           C.byref(g), C.byref(he), C.byref(m)), None)
+        return g.value, he.value, bool(m.value)
+
+    def stats(self):
+        r, b, u = C.c_int64(), C.c_int64(), C.c_int64()
+        _check(lib().cds_shape_pairq_get_stats(self.h, C.byref(r), C.byref(b), C.byref(u)), None)
+        return {"requests": r.value, "batches": b.value, "uploads": u.value}
+
+    def drive(self, targets_rgb, gradients, zgaps_rgb, keys, pair_mask, pair_target, n_threads):
+        """n_threads native threads call cds_shape_pairq_score over the pair list -> (gap, high_expr, mirrored, seconds)"""
+        targets_rgb = np.ascontiguousarray(targets_rgb, dtype=np.uint8)
+        gradients = np.ascontiguousarray(gradients, dtype=np.uint16)
+        zgaps_rgb = None if zgaps_rgb is None else np.ascontiguousarray(zgaps_rgb, dtype=np.uint8)
+        assert gradients.shape[0] == targets_rgb.shape[0] and (zgaps_rgb is None or zgaps_rgb.shape == targets_rgb.shape)
+        keys = None if keys is None else np.ascontiguousarray(keys, dtype=np.uint64)
+        pair_mask = np.ascontiguousarray(pair_mask, dtype=np.int32)
+        pair_target = np.ascontiguousarray(pair_target, dtype=np.int64)
+        n = len(pair_mask)
+        gap = np.zeros(n, np.int64)
+        he = np.zeros(n, np.int64)
+        mir = np.zeros(n, np.uint8)
+        secs = C.c_double()
+        _check(lib().cds_debug_shape_pairq_drive(self.h, _ptr(targets_rgb), _ptr(gradients), _ptr(zgaps_rgb), targets_rgb.shape[0],
+                                                 None if keys is None else keys.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                 pair_mask.ctypes.data_as(_i32p), pair_target.ctypes.data_as(_i64p), n, int(n_threads),
+                                                 gap.ctypes.data_as(_i64p), he.ctypes.data_as(_i64p), mir.ctypes.data_as(_u8p), C.byref(secs)), None)
+        return gap, he, mir.astype(bool), secs.value
 
 
 def shape_score_2d(gap, he):

@@ -37,6 +37,7 @@
 
 #include "cds_lut.h"
 #include "cds_runtime.h"
+#include "cds_shape.cuh"
 #include "cds_tiff.h"
 
 using namespace cds;
@@ -638,13 +639,6 @@ __global__ void __launch_bounds__(256) shape_roi_bits_kernel(const uint8_t *__re
 }
 
 // ------------------------------------------------------------------------------------------------------------------ pair kernel
-struct ShapeMaskDesc {
-    const uint32_t *gap_list;
-    const uint32_t *he_n, *he_m;
-    int n_gap;
-    int pad;
-};
-
 // pair_slot = index of the pair's target inside the window's planes
 __global__ void __launch_bounds__(256) shape_pair_kernel(const ShapeMaskDesc *__restrict__ masks, const int32_t *__restrict__ pair_mask,
                                                          const int32_t *__restrict__ pair_slot,
@@ -660,33 +654,9 @@ __global__ void __launch_bounds__(256) shape_pair_kernel(const ShapeMaskDesc *__
     const uint16_t *gr = grad + (size_t) t * W * H;
     const uint32_t *ts = tsig + (size_t) t * H * bpitch;
     long long gap_n = 0, gap_m = 0, he_n = 0, he_m = 0;
-    for (int i = threadIdx.x; i < md.n_gap; i += blockDim.x) {
-        const uint32_t e = __ldg(md.gap_list + i);
-        const int x = (int) (e & 0x7FFu), y = (int) ((e >> 11) & 0x3FFu);
-        const int qs = (int) ((e >> 21) & 0xFFu) + 1;
-        const int qm = (int) ((e >> 29) & 1u);
-        const size_t rowoff = (size_t) y * W;
-        const int z = zs[rowoff + x];                            // the zgap image is sampled at the query's own pixel in both orientations
-        int big = 0;
-        if (z != 0) {                                            // PIXEL_GAP_OP :30-37
-            const int pxGapSlice = abs(qs - z);
-            if (40 <= pxGapSlice - 40) big = pxGapSlice - 40;
-        }
-        if (e & 0x40000000u) {
-            const int gap = big ? big : qm * (int) gr[rowoff + x];
-            if (gap > 3) gap_n += gap;
-        }
-        if (mirror && (e & 0x80000000u)) {
-            const int gap = big ? big : qm * (int) gr[rowoff + (W - 1 - x)];   // the gradient is NOT mirrored with the query :222
-            if (gap > 3) gap_m += gap;
-        }
-    }
+    for (int i = threadIdx.x; i < md.n_gap; i += blockDim.x) shape_gap_entry(__ldg(md.gap_list + i), zs, gr, W, mirror, gap_n, gap_m);
     const int n_words = H * bpitch;
-    for (int i = threadIdx.x; i < n_words; i += blockDim.x) {
-        const uint32_t tw = ts[i];
-        he_n += __popc(__ldg(md.he_n + i) & tw);
-        if (mirror) he_m += __popc(__ldg(md.he_m + i) & tw);
-    }
+    for (int i = threadIdx.x; i < n_words; i += blockDim.x) shape_he_word(md, ts, i, mirror, he_n, he_m);
     long long v[4] = {gap_n, gap_m, he_n, he_m};
 #pragma unroll
     for (int k = 0; k < 4; k++) {
@@ -698,14 +668,8 @@ __global__ void __launch_bounds__(256) shape_pair_kernel(const ShapeMaskDesc *__
     if (threadIdx.x == 0) {
         long long tot[4] = {0, 0, 0, 0};
         for (int k = 0; k < 4; k++) for (int w = 0; w < 8; w++) tot[k] += s_red[k][w];
-        long long g = tot[0], h = tot[2];
-        int mir = 0;
-        if (mirror) {
-            // ShapeMatchScore.getScore narrows calculate2DShapeScore to int; mirrored wins when strictly smaller (:181)
-            const int s0 = (int) (tot[0] + tot[2] / 3);
-            const int s1 = (int) (tot[1] + tot[3] / 3);
-            if (s1 < s0) { g = tot[1]; h = tot[3]; mir = 1; }
-        }
+        long long g, h;
+        const int mir = shape_pick(tot, mirror, g, h);
         gap_out[pr] = g; he_out[pr] = h; mir_out[pr] = (uint8_t) mir;
     }
 }
@@ -762,26 +726,21 @@ static bool launch_target_derive(const uint8_t *target, int64_t n, int W, int H,
 }  // namespace cds
 
 // ------------------------------------------------------------------------------------------------------------------ C ABI
-struct cds_shape_maskset {
-    cds_ctx *ctx = nullptr;
-    int W = 0, H = 0, bpitch = 0;
-    int query_threshold = 0, mirror = 0;
-    RectSet rects{};
-    uint32_t *d_roi_bits = nullptr;                  // label-cleared ROI bitmap on device 0 (where masks are prepared), or nullptr
-    int n_masks = 0;
-    // per device: the masks' descriptors (device-local pointers), the blocks that hold their lists and bitmaps
-    struct Dev {
-        std::vector<ShapeMaskDesc> h_descs;
-        std::vector<void *> blocks;
-        ShapeMaskDesc *d_descs = nullptr;
-        size_t d_descs_cap = 0;
-        bool dirty = true;
-    };
-    std::vector<Dev> dev;
-};
-
 #define SH_TRY(expr) do { cds_status _s = (expr); if (_s != CDS_OK) return _s; } while (0)
 #define SH_CUDA(ctx, expr) SH_TRY((ctx)->check((expr), #expr))
+
+void cds::launch_shape_target_planes(const cds_shape_maskset *sms, const DevState &ds, const uint8_t *target, const uint8_t *zgap, int64_t n,
+                                     uint16_t *zslice, uint32_t *tsig, cudaStream_t s)
+{
+    if (zgap) {
+        target_planes_kernel<<<dim3(sms->H, (unsigned) n), 256, 0, s>>>(target, zgap, sms->W, sms->H, sms->rects, sms->query_threshold, sms->bpitch,
+                                                                       ds.d_slice_tab, zslice, tsig);
+    } else {
+        // the zgap image the reference's tests derive: maxFilter(10)(mask(threshold)(clearLabels(target))), never materialised
+        launch_target_derive<false>(target, n, sms->W, sms->H, sms->rects, sms->query_threshold, make_disc(10), ds.d_slice_tab, zslice, tsig,
+                                    sms->bpitch, nullptr, s);
+    }
+}
 
 static RectSet to_rectset(const cds_rect *rects, int n)
 {
@@ -1119,7 +1078,6 @@ static cds_status shape_score_pairs_impl(cds_ctx *ctx, const cds_shape_maskset *
     }
     const int64_t n_windows = ((int64_t) active.size() + win - 1) / win;
     const int used = (int) std::min<int64_t>(D, n_windows);
-    const DiscSpec disc10 = make_disc(10);
 
     // window w -> device w % used; per device the pairs of its windows in window order
     std::vector<ShapeDevWork> work(used);
@@ -1365,14 +1323,7 @@ static cds_status shape_score_pairs_impl(cds_ctx *ctx, const cds_shape_maskset *
                 }
                 if (st != CDS_OK) break;
             }
-            if (zgap_rgb) {
-                target_planes_kernel<<<dim3(H, (unsigned) cnt), 256, 0, ds.stream>>>(wk.d_t[slot], wk.d_z[slot], W, H, sms->rects, sms->query_threshold, bpitch,
-                                                                                    ds.d_slice_tab, wk.d_zslice, wk.d_tsig);
-            } else {
-                // the zgap image the reference's tests derive: maxFilter(10)(mask(threshold)(clearLabels(target))), never materialised
-                launch_target_derive<false>(wk.d_t[slot], cnt, W, H, sms->rects, sms->query_threshold, disc10, ds.d_slice_tab, wk.d_zslice, wk.d_tsig, bpitch,
-                                            nullptr, ds.stream);
-            }
+            launch_shape_target_planes(sms, ds, wk.d_t[slot], zgap_rgb ? wk.d_z[slot] : nullptr, cnt, wk.d_zslice, wk.d_tsig, ds.stream);
             ctx->stats.kernel_launches++;
             const auto pr = win_pairs[d][j];
             cudaEventRecord(ds.shape_timing[2 * j], ds.stream);

@@ -387,6 +387,34 @@ cds_status cds_shape_score_pairs_files(cds_ctx *ctx, const cds_shape_maskset *sm
                                        const int32_t *pair_mask, const int64_t *pair_target, int64_t n_pairs,
                                        int64_t *gap_out, int64_t *high_expr_out, uint8_t *mirrored_out);
 
+/* The shape score's single-pair call at scale: a micro-batching scorer with a device-side cache of derived target planes.
+ * gradientScores makes one Shape2DMatchColorDepthSearchAlgorithm.calculateMatchingScore(target, variantSuppliers) call per (mask, target)
+ * pair (API/cds/Shape2DMatchColorDepthSearchAlgorithm.java:150-245) from a thread pool (TOOLS/CalculateGradientScoresCmd.java:304-312),
+ * and the same target recurs across masks.  cds_shape_pairq_score is that call: it blocks its caller until the pair is scored, may be
+ * called from any number of threads at once and does not take the context's lock; calls that arrive together are scored by one kernel
+ * launch, and a target whose key is already cached is neither uploaded nor derived again.  Returns what cds_shape_score_pairs returns
+ * for the same pair, bit for bit.
+ *   max_batch, max_wait_us, target_key   as for cds_pairq (several queues per device, environment CDSGPU_PAIRQ_QUEUES); equal keys MUST
+ *                 mean equal target, gradient and zgap pixels and the same choice of given or derived zgap image; key 0 = do not cache
+ *   cache_targets derived targets kept on every device (at least 2 * max_batch per queue); a slot holds the slice plane, the gradient and
+ *                 the signal bitmap: 2 * W * H * 2 + H * bpitch * 4 bytes with bpitch = ceil(W / 32) rounded up to a multiple of 4
+ *                 (2.83 MB at 1210 x 566); least recently used are replaced
+ *   gradient      uint16[H][W]; NULL = the gradient supplier is missing: (-1, -1, 0) and CDS_OK, no device work (:155-158)
+ *   zgap_rgb      uint8[H][W][3] or NULL = derived on the device as in cds_shape_score_pairs
+ * Masks may be ADDED to the shape mask set while the queue exists: the first call that names a new mask pauses the dispatchers
+ * between two batches and picks the new masks up.  The mask set must not be destroyed before the queue.  CDS_ERR_SIZE_MISMATCH for a
+ * target of another size, CDS_ERR_BAD_ARG for a mask index out of range or a NULL target with a gradient. */
+typedef struct cds_shape_pairq cds_shape_pairq;
+cds_status cds_shape_pairq_create(cds_ctx *ctx, const cds_shape_maskset *sms, int32_t max_batch, int32_t max_wait_us,
+                                  int32_t cache_targets, cds_shape_pairq **out);
+void       cds_shape_pairq_destroy(cds_shape_pairq *q);
+cds_status cds_shape_pairq_score(cds_shape_pairq *q, int32_t mask_index, uint64_t target_key,
+                                 const uint8_t *target_rgb, const uint16_t *gradient, const uint8_t *zgap_rgb,
+                                 int32_t target_width, int32_t target_height,
+                                 int64_t *gap_out, int64_t *high_expr_out, int32_t *mirrored_out);
+/* requests served, kernel launches (batches) and target uploads so far (any pointer may be NULL) */
+cds_status cds_shape_pairq_get_stats(const cds_shape_pairq *q, int64_t *requests, int64_t *batches, int64_t *uploads);
+
 /* The zgap image alone (f3 in SURVEY.md section 8f): maxFilter(radius)(mask(threshold)(clearLabels(rgb))) for n images. */
 cds_status cds_make_zgap(cds_ctx *ctx, const uint8_t *rgb, int64_t n, int32_t width, int32_t height, int32_t threshold,
                          double radius, const cds_rect *rects, int32_t n_rects, uint8_t *zgap_out);
@@ -541,6 +569,13 @@ cds_status cds_debug_stream_plan(int32_t n_devices, int64_t n_targets, int64_t c
 cds_status cds_debug_pairq_drive(cds_pairq *q, const uint8_t *targets_rgb, int64_t n_targets, const uint64_t *keys,
                                  const int32_t *pair_mask, const int64_t *pair_target, int64_t n_pairs, int32_t n_threads,
                                  int32_t *scores_out, uint8_t *mirrored_out, double *seconds_out);
+/* Drives cds_shape_pairq_score from n_threads native threads over a list of pairs, like cds_debug_pairq_drive: target t is
+ * targets_rgb[t], gradients[t] and zgaps_rgb[t] (zgaps_rgb may be NULL: derived) with key keys[t] (keys may be NULL: 0).
+ * seconds_out = wall clock of the whole run. */
+cds_status cds_debug_shape_pairq_drive(cds_shape_pairq *q, const uint8_t *targets_rgb, const uint16_t *gradients,
+                                       const uint8_t *zgaps_rgb, int64_t n_targets, const uint64_t *keys,
+                                       const int32_t *pair_mask, const int64_t *pair_target, int64_t n_pairs, int32_t n_threads,
+                                       int64_t *gap_out, int64_t *high_expr_out, uint8_t *mirrored_out, double *seconds_out);
 /* Slice numbers (1..256, 0 = black) of n RGB colours as the shape path computes them on the device -- a table built per device
  * with the double arithmetic of GradientAreaGapUtils.findSliceNumberInLUT (API/cds/GradientAreaGapUtils.java:18-197) -- so that the
  * table can be checked against the oracle over all 2^24 colours. */

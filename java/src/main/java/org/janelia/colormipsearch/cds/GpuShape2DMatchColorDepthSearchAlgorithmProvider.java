@@ -19,6 +19,13 @@ import org.janelia.colormipsearch.model.ComputeFileType;
 /**
  * Drop-in for createShapeMatchCDSAlgorithmProvider (ColorDepthSearchAlgorithmProviderFactory.java:76-127).  Lives in package
  * org.janelia.colormipsearch.cds because ShapeMatchScore's constructors are package-private (ShapeMatchScore.java:12,20).
+ *
+ * Every calculateMatchingScore is one blocking cds_shape_pairq_score call.  The calls of gradientScores' pool threads
+ * (CalculateGradientScoresCmd.java:304-312) meet in the library's micro-batching queue and are scored by one kernel launch per batch;
+ * a target that was scored before is found in the device-side cache of derived planes by its identity (the same key as the pixel
+ * provider's), so it is uploaded and derived once.  All algorithms of one parameter set share ONE native shape mask set and ONE queue
+ * (masks are appended as algorithms are created).
+ *
  * UNVERIFIED (no JDK in the build image of the GPU library).
  */
 public class GpuShape2DMatchColorDepthSearchAlgorithmProvider implements ColorDepthSearchAlgorithmProvider<ShapeMatchScore> {
@@ -34,33 +41,61 @@ public class GpuShape2DMatchColorDepthSearchAlgorithmProvider implements ColorDe
 
     @Override public ColorDepthSearchParams getDefaultCDSParams() { return defaults; }
 
+    /** One native shape mask set + pair queue per (image size, query threshold, border, mirror, excluded rectangles). */
+    private static final class Shared {
+        MemorySegment maskSet, queue;
+        int nMasks;
+    }
+    private final Map<String, Shared> shared = new java.util.HashMap<>();
+
+    private synchronized int addMask(String key, ImageArray<?> queryImage, int queryThreshold, int border, boolean mirror, int[][] rects,
+                                     Shared[] out, int[] sizeOut) {
+        Shared sh = shared.get(key);
+        try (Arena a = Arena.ofConfined()) {
+            MemorySegment o = a.allocate(ValueLayout.ADDRESS), qm = a.allocate(ValueLayout.JAVA_LONG), he = a.allocate(ValueLayout.JAVA_LONG);
+            if (sh == null) {
+                sh = new Shared();
+                MemorySegment r = a.allocate(16L * Math.max(rects.length, 1));
+                for (int i = 0; i < rects.length; i++) for (int k = 0; k < 4; k++) r.set(ValueLayout.JAVA_INT, 16L * i + 4L * k, rects[i][k]);
+                MemorySegment roiSeg = roiMask == null ? MemorySegment.NULL : CdsGpu.copyBytes(a, ImageArrayAccess.rgbBytes(roiMask));
+                CdsGpu.check((int) CdsGpu.shapeMasksetCreate.invokeExact(CdsGpu.context(), queryImage.getWidth(), queryImage.getHeight(), queryThreshold, border,
+                        mirror ? 1 : 0, r, rects.length, roiSeg, o));
+                sh.maskSet = o.get(ValueLayout.ADDRESS, 0);
+                shared.put(key, sh);
+            }
+            CdsGpu.check((int) CdsGpu.shapeMasksetAddRgb.invokeExact(sh.maskSet, CdsGpu.copyBytes(a, ImageArrayAccess.rgbBytes(queryImage)), 1, qm, he));
+            sizeOut[0] = (int) qm.get(ValueLayout.JAVA_LONG, 0);
+            if (sh.queue == null) {
+                // max batch 256, wait at most 60 us for company, 1024 derived targets per device (2.9 GB for 1210 x 566)
+                CdsGpu.check((int) CdsGpu.shapePairqCreate.invokeExact(CdsGpu.context(), sh.maskSet, 256, 60, Integer.getInteger("cdsgpu.cachedShapeTargets", 1024), o));
+                sh.queue = o.get(ValueLayout.ADDRESS, 0);
+            }
+            out[0] = sh;
+            return sh.nMasks++;
+        } catch (RuntimeException e) { throw e; } catch (Throwable t) { throw new IllegalStateException(t); }
+    }
+
     @Override
     public ColorDepthSearchAlgorithm<ShapeMatchScore> createColorDepthSearchAlgorithm(ImageArray<?> queryImage, int queryThreshold,
                                                                                       int queryBorderSize, ColorDepthSearchParams cdsParams) {
         boolean mirror = cdsParams.getBoolParam("mirrorMask", defaults.getBoolParam("mirrorMask", false));
         int[][] rects = GpuPixelMatchColorDepthSearchAlgorithmProvider.rectanglesOf(excludedRegions, queryImage);
-        return new Algorithm(queryImage, queryThreshold, queryBorderSize, mirror, roiMask, rects);
+        String key = queryImage.getWidth() + "x" + queryImage.getHeight() + ":" + queryThreshold + ":" + queryBorderSize + ":" + mirror
+                + ":" + java.util.Arrays.deepToString(rects);
+        Shared[] sh = new Shared[1];
+        int[] size = new int[1];
+        int index = addMask(key, queryImage, queryThreshold, queryBorderSize, mirror, rects, sh, size);
+        return new Algorithm(queryImage, sh[0].queue, index, size[0]);
     }
 
     static final class Algorithm implements ColorDepthSearchAlgorithm<ShapeMatchScore> {
         private static final Set<ComputeFileType> REQUIRED = EnumSet.of(ComputeFileType.GradientImage, ComputeFileType.ZGapImage);
         private final ImageArray<?> queryImage;
-        private final transient MemorySegment shapeMaskSet;
-        private final int querySize;
+        private final transient MemorySegment queue;   // native handle: not serialisable, Spark mode is unsupported on this provider
+        private final int maskIndex, querySize;
 
-        Algorithm(ImageArray<?> queryImage, int queryThreshold, int border, boolean mirror, ImageArray<?> roi, int[][] rects) {
-            this.queryImage = queryImage;
-            try (Arena a = Arena.ofConfined()) {
-                MemorySegment out = a.allocate(ValueLayout.ADDRESS), qm = a.allocate(ValueLayout.JAVA_LONG), he = a.allocate(ValueLayout.JAVA_LONG);
-                MemorySegment r = a.allocate(16L * Math.max(rects.length, 1));
-                for (int i = 0; i < rects.length; i++) for (int k = 0; k < 4; k++) r.set(ValueLayout.JAVA_INT, 16L * i + 4L * k, rects[i][k]);
-                MemorySegment roiSeg = roi == null ? MemorySegment.NULL : CdsGpu.copyBytes(a, ImageArrayAccess.rgbBytes(roi));
-                CdsGpu.check((int) CdsGpu.shapeMasksetCreate.invokeExact(CdsGpu.context(), queryImage.getWidth(), queryImage.getHeight(), queryThreshold, border,
-                        mirror ? 1 : 0, r, rects.length, roiSeg, out));
-                shapeMaskSet = out.get(ValueLayout.ADDRESS, 0);
-                CdsGpu.check((int) CdsGpu.shapeMasksetAddRgb.invokeExact(shapeMaskSet, CdsGpu.copyBytes(a, ImageArrayAccess.rgbBytes(queryImage)), 1, qm, he));
-                querySize = (int) qm.get(ValueLayout.JAVA_LONG, 0);
-            } catch (RuntimeException e) { throw e; } catch (Throwable t) { throw new IllegalStateException(t); }
+        Algorithm(ImageArray<?> queryImage, MemorySegment queue, int maskIndex, int querySize) {
+            this.queryImage = queryImage; this.queue = queue; this.maskIndex = maskIndex; this.querySize = querySize;
         }
 
         @Override public ImageArray<?> getQueryImage() { return queryImage; }
@@ -69,6 +104,7 @@ public class GpuShape2DMatchColorDepthSearchAlgorithmProvider implements ColorDe
         @Override public int getQueryLastPixelIndex() { return queryImage.getPixelCount() - 1; }
         @Override public Set<ComputeFileType> getRequiredTargetVariantTypes() { return REQUIRED; }
 
+        /** Thread-safe and re-entrant: cds_shape_pairq_score takes no context-wide lock; calls that arrive together share a kernel launch. */
         @Override
         public ShapeMatchScore calculateMatchingScore(@Nonnull ImageArray<?> target, Map<ComputeFileType, Supplier<ImageArray<?>>> variants) {
             ImageArray<?> grad = fetch(variants, ComputeFileType.GradientImage), zgap = fetch(variants, ComputeFileType.ZGapImage);
@@ -78,12 +114,12 @@ public class GpuShape2DMatchColorDepthSearchAlgorithmProvider implements ColorDe
                 MemorySegment g16 = a.allocate(2L * n, 2);
                 if (ImageArrayAccess.isGray16(grad)) MemorySegment.copy(ImageArrayAccess.gray16(grad), 0, g16, ValueLayout.JAVA_SHORT, 0, n);
                 else { byte[] g8 = ImageArrayAccess.gray8(grad); for (int i = 0; i < n; i++) g16.set(ValueLayout.JAVA_SHORT, 2L * i, (short) (g8[i] & 0xFF)); }
-                MemorySegment pm = a.allocate(ValueLayout.JAVA_INT), pt = a.allocate(ValueLayout.JAVA_LONG);
-                MemorySegment gap = a.allocate(ValueLayout.JAVA_LONG), he = a.allocate(ValueLayout.JAVA_LONG), mir = a.allocate(ValueLayout.JAVA_BYTE);
-                CdsGpu.check((int) CdsGpu.shapeScorePairs.invokeExact(CdsGpu.context(), shapeMaskSet,
+                MemorySegment gap = a.allocate(ValueLayout.JAVA_LONG), he = a.allocate(ValueLayout.JAVA_LONG), mir = a.allocate(ValueLayout.JAVA_INT);
+                // the key is the target ImageArray's identity: its gradient and zgap images come with it
+                CdsGpu.check((int) CdsGpu.shapePairqScore.invokeExact(queue, maskIndex, GpuPixelMatchColorDepthSearchAlgorithmProvider.targetKey(target),
                         CdsGpu.copyBytes(a, ImageArrayAccess.rgbBytes(target)), g16, CdsGpu.copyBytes(a, ImageArrayAccess.rgbBytes(zgap)),
-                        MemorySegment.NULL, 1L, pm, pt, 1L, gap, he, mir));
-                return new ShapeMatchScore(gap.get(ValueLayout.JAVA_LONG, 0), he.get(ValueLayout.JAVA_LONG, 0), -1, mir.get(ValueLayout.JAVA_BYTE, 0) != 0);
+                        target.getWidth(), target.getHeight(), gap, he, mir));
+                return new ShapeMatchScore(gap.get(ValueLayout.JAVA_LONG, 0), he.get(ValueLayout.JAVA_LONG, 0), -1, mir.get(ValueLayout.JAVA_INT, 0) != 0);
             } catch (RuntimeException e) { throw e; } catch (Throwable t) { throw new IllegalStateException(t); }
         }
 

@@ -81,6 +81,10 @@ public final class CdsGpu {
     public static final MethodHandle shapeMasksetDestroy = h("cds_shape_maskset_destroy", FunctionDescriptor.ofVoid(ADDRESS));
     public static final MethodHandle shapeMasksetAddRgb = h("cds_shape_maskset_add_rgb", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, ADDRESS));
     public static final MethodHandle shapeScorePairs = h("cds_shape_score_pairs", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS));
+    // the shape score's single-pair call behind a micro-batching queue with a device-side cache of derived target planes (cds_shape_pairq_*)
+    public static final MethodHandle shapePairqCreate = h("cds_shape_pairq_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS));
+    public static final MethodHandle shapePairqDestroy = h("cds_shape_pairq_destroy", FunctionDescriptor.ofVoid(ADDRESS));
+    public static final MethodHandle shapePairqScore = h("cds_shape_pairq_score", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS, ADDRESS, ADDRESS));
 
     /** One context per JVM: the lifetime of a command run (colorDepthSearch / gradientScores). */
     private static volatile MemorySegment CTX;
